@@ -13,6 +13,7 @@ One JSON line is printed by rank 0.
 from __future__ import annotations
 
 import argparse
+import copy
 import json
 import os
 import statistics
@@ -49,7 +50,16 @@ def parse_args():
                          "(name, stream, start_us, dur_us) and exit -- a diagnostic, never a bench value")
     ap.add_argument("--ncu-step", action="store_true",
                     help="warm up, then run ONE step between cudaProfilerStart/Stop and exit (use with ncu --profile-from-start off)")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the measurements, run one more step of the timed path from the seeded initial weights and "
+                         "optimizer state and write what it computed (loss, loss terms, evaluator metrics, updated parameters, a "
+                         "fixed sample of the gradients; c5: the tokens of the last timed call) as DIR/<name>.npy, so two builds "
+                         "can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs covers the timed path of --impl b200")
     if args.batch is None:
         args.batch = 64 if args.config == "c2" else 16
     if args.seq is None:
@@ -118,14 +128,12 @@ def algorithmic_flops_per_tuple(T: int) -> float:
 
 
 # ----------------------------------------------------------------------------- reference arm / CPU baseline
-# The UNMODIFIED reference lives in baseline/_ref (copied there by __graft_entry__.build(); git-ignored, shipped with the
-# snapshot) and is driven through oracle/ref_shim.py, which only supplies stand-ins for the absent omegaconf / miditok imports.
-# If it is not there (a checkout that never ran build() next to /root/reference) the oracle port is timed instead, kind "port".
+# The UNMODIFIED reference is a copy of the original project found by tests/parity.reference_root() ($SPB200_REFERENCE_ROOT, else
+# baseline/_ref), driven through oracle/ref_shim.py, which only supplies stand-ins for the absent omegaconf / miditok imports.
+# Without one the oracle port is timed instead, kind "port".
 def _reference_root():
-    for cand in (os.path.join(ROOT, "baseline", "_ref"), "/root/reference"):
-        if os.path.isdir(os.path.join(cand, "scoreperformer")) and os.path.isdir(os.path.join(cand, "recipes")):
-            return cand
-    return None
+    from tests.parity import reference_root
+    return reference_root()
 
 
 def build_reference(device: str = "cpu"):
@@ -217,6 +225,49 @@ def workload_config(B, T, world, graph=True):
             "l2": "per-step activations (>3 GB) far exceed the 126 MB L2; no explicit flush needed"}
 
 
+DUMP_GRAD_SAMPLES = 1 << 20
+DUMP_MAX_BYTES = 64_000_000
+
+
+def step_outputs(model, ts, loss):
+    """Host copies of what a caller has after a training step: the loss, its terms and the evaluator's metrics, every parameter
+    as updated by the step, and the gradients at 2^20 fixed positions (drawn with seed 0 from the parameters' gradients
+    concatenated in registration order, so the sample does not depend on how the step lays out its buffers)."""
+    def host(t):
+        t = torch.as_tensor(t).detach().cpu()
+        return (t.double() if t.dtype == torch.float64 else t.float()).numpy()
+    out = {"loss": host(loss)}
+    out.update({f"losses.{k}": host(v) for k, v in ts.losses.items()})
+    out.update({f"metrics.{k}": host(v) for k, v in (ts.metrics or {}).items()})
+    params = [(k, p) for k, p in model.named_parameters() if p.grad is not None]
+    out.update({f"param.{k}": host(p) for k, p in params})
+    grads = torch.cat([p.grad.detach().reshape(-1) for _, p in params])
+    idx = torch.randint(grads.numel(), (DUMP_GRAD_SAMPLES,), generator=torch.Generator().manual_seed(0)).sort().values
+    out["grad_sample"] = host(grads[idx.to(grads.device)])
+    return out
+
+
+def step_from(model, ts, initial, batch):
+    """One step of the timed path (captured afresh for the restored state, then replayed) from `initial` = (model state_dict,
+    optimizer state) on `batch`, and its outputs (step_outputs)."""
+    sd, opt = initial
+    model.load_state_dict(sd)
+    ts.load_optimizer_state_dict(opt)                    # also drops the captured graphs
+    ts.mark_weights_changed()
+    return step_outputs(model, ts, ts.step(batch))
+
+
+def write_outputs(directory, outputs):
+    """One DIR/<name>.npy per array ('/' in loss and metric names becomes '.')."""
+    total = sum(a.nbytes for a in outputs.values())
+    if total > DUMP_MAX_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes of outputs exceed the {DUMP_MAX_BYTES}-byte budget")
+    os.makedirs(directory, exist_ok=True)
+    import numpy as np
+    for name, a in outputs.items():
+        np.save(os.path.join(directory, name.replace("/", ".") + ".npy"), a)
+
+
 def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
@@ -246,8 +297,7 @@ def main():
         return
     if args.config == "c5":
         import bench_render
-        sys.argv = [sys.argv[0]]
-        bench_render.main()
+        bench_render.main([] if args.dump_outputs is None else ["--dump-outputs", args.dump_outputs])
         return
 
     import torch.distributed as dist
@@ -273,6 +323,9 @@ def main():
     model.perf_encoder.exact_latent_shapes = False          # static segment tables: no host sync inside the step
     model.perf_decoder.label_fields = (3, 5, 10, 11)        # MixedLM collator labels (base.yaml:64-65): no probe sync
     ts = TrainStep(model, lr=2e-4, weight_decay=1e-6, grad_clip=2.0, use_graph=not args.no_graph)
+    # the seeded starting point of the step --dump-outputs replays: the weights every later step starts from carry the rounding of
+    # the earlier steps' atomic reductions (their order varies from run to run), so only this state is the same in every run
+    initial = (copy.deepcopy(model.state_dict()), ts.optimizer_state_dict()) if args.dump_outputs else None
     # the reference trainer evaluates its metrics after every training step (experiments/trainer.py:462-464, recipe settings
     # base.yaml:195-198): the timed step does too -- the head kernel accumulates the statistics, the evaluator divides
     from scoreperformer_b200.models.scoreperformer.evaluator import ScorePerformerEvaluator
@@ -511,6 +564,11 @@ def main():
             "reference_gpu": reference_gpu,
         }
         print(json.dumps(line), flush=True)
+    if initial is not None:
+        ts.use_graph = not args.no_graph                 # the roofline pass above switched to eager steps
+        outputs = step_from(model, ts, initial, dev_batch)
+        if rank == 0:
+            write_outputs(args.dump_outputs, outputs)
     if world > 1:
         ts.close()                       # the captured graphs hold NCCL kernels: release them before the communicator goes
         dist.barrier()

@@ -13,12 +13,14 @@ sys.path.insert(0, os.path.join(ROOT, "oracle"))
 import torch  # noqa: E402
 
 
-def main():
+def main(argv=None):
     ap = argparse.ArgumentParser()
     ap.add_argument("--scores", type=int, default=256)
     ap.add_argument("--notes", type=int, default=1024)
     ap.add_argument("--cpu-notes", type=int, default=48)
-    args = ap.parse_args()
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the tokens the last timed call rendered as DIR/tokens.npy (float32: the ids are exact)")
+    args = ap.parse_args(argv)
     from tests import parity
     from scoreperformer_b200 import kernels as K
     from scoreperformer_b200.decode import render_batch
@@ -48,6 +50,10 @@ def main():
             torch.cuda.synchronize()
             times.append(time.perf_counter() - t0)
         dt_cold, dt = times[0], min(times[1:])
+    if args.dump_outputs:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "tokens.npy"), out.cpu().numpy().astype(np.float32))
     notes = B * (T - 1)
     # CPU reference: batch-1 cached greedy loop of the oracle port on a short score
     import model_oracle as mo

@@ -208,6 +208,99 @@ def random_chunks(seed: int, n_notes: int = 160, metre_change: bool = False):
     return piece, cuts
 
 
+# ----------------------------------------------------------------------------- seeded random cases (tests/golden/inference_live.npz)
+# Each function drives one side (`arm`) through a fixed list of random cases and returns a flat {key: array} record; the tests
+# compare this package's record with the stored one and, where a copy of the original project is supplied, with the original's.
+def fuzz_scenarios():
+    """14 random rendering scenarios (default_rng(2024)): name -> (SCENARIOS entry, SPMuple2 family?).  Every fifth one uses the
+    SPMuple family (tick-based messenger, no tempo state)."""
+    rng = np.random.default_rng(2024)
+    out = {}
+    for i in range(14):
+        params = [{}, dict(decode_recompute_tempos=False), dict(onset_tempos=True), dict(use_quantized_tempos=False, tempo_window=3.)][i % 4]
+        ignore = (0, 1, 2, 4, 6, 7, 8, 9) if i % 3 else (0, 1, 2, 4, 5, 6, 7, 8, 9)
+        gen_kw = dict(max_context_len=int(rng.choice([24, 40, 64, 512])), group_chord_notes=bool(rng.random() < 0.7),
+                      time_window_overflow=float(rng.choice([0., 0.1, 0.3])), disable_caches=bool(rng.random() < 0.2),
+                      delta=bool(rng.random() < 0.4), sort_messages=bool(rng.random() < 0.5))
+        entry = (dict(n_notes=int(rng.integers(40, 160)), seed=int(rng.integers(1000))), params, ignore, gen_kw,
+                 float(rng.choice([0.25, 0.5, 1.0, 2.5])), "spm2")
+        out[f"fuzz{i}"] = (entry, i % 5 != 4)
+    return out
+
+
+def run_fuzz_renderings(arm):
+    """`arm(spm2, params)` -> (generator class, messenger class, tokenizer, cache classes, intermediates class).  Each field of the
+    windows is stored concatenated over them, with its row count per window."""
+    out = {}
+    for name, (entry, spm2) in fuzz_scenarios().items():
+        SCENARIOS[name] = entry
+        try:
+            windows, final = run_scenario(name, *arm(spm2, entry[1]))
+        finally:
+            SCENARIOS.pop(name)
+        for k in windows[0]:
+            parts = [np.atleast_2d(w[k]) if w[k].ndim < 2 else w[k] for w in windows]
+            out[f"{name}/{k}"] = np.concatenate(parts)
+            out[f"{name}/{k}_rows"] = np.array([len(p) for p in parts], dtype=np.int64)
+        for k, v in final.items():
+            out[f"{name}/final/{k}"] = v
+    return out
+
+
+def run_messenger_configurations(arm):
+    """16 random messenger settings (default_rng(77)) with metre changes and chunkings; `arm(spm2, params)` -> messenger.  Per case:
+    the messages of every chunk (SPMuple: also its tick messages) concatenated, the tempo map and the onset pairs carried at the end."""
+    rng = np.random.default_rng(77)
+    out = {}
+    for i in range(16):
+        spm2 = i % 2 == 0
+        params = dict(decode_recompute_tempos=bool(rng.random() < 0.6), onset_tempos=bool(rng.random() < 0.25),
+                      use_quantized_tempos=bool(rng.random() < 0.5), tempo_window=float(rng.choice([1., 4., 8., 1e6])),
+                      tempo_min_onsets=int(rng.choice([2, 8, 40])), tempo_min_onset_dist=float(rng.choice([0.1, 0.5, 2.])),
+                      bar_tempos=bool(rng.random() < 0.5), use_position_shifts=bool(rng.random() < 0.5),
+                      onset_position_shifts=bool(rng.random() < 0.5), rel_onset_dev=True, rel_perf_duration=bool(spm2 or rng.random() < 0.7))
+        if not spm2 and not params["rel_perf_duration"]:
+            continue                                       # absolute PerfDuration needs its own vocabulary column
+        m = arm(spm2, params)
+        piece, cuts = random_chunks(int(rng.integers(10000)), n_notes=int(rng.integers(30, 400)), metre_change=bool(rng.random() < 0.4))
+        state, lo, msgs = None, 0, []
+        for hi in cuts:
+            if not spm2:
+                msgs.append(m.tokens_to_messages(piece[lo:hi].copy(), intermediates=state, to_times=False, sort=True))
+            chunk_msgs, state = m.tokens_to_messages(piece[lo:hi].copy(), intermediates=state, return_intermediates=True, sort=bool(hi % 2))
+            msgs.append(chunk_msgs)
+            lo = hi
+        out[f"case{i}/messages"] = np.concatenate(msgs)
+        out[f"case{i}/tempos"] = np.asarray(state.tempos, dtype=np.float64)
+        out[f"case{i}/pairs"] = np.asarray(getattr(state, "onset_pairs", None) if spm2 else [[0.]], dtype=np.float64)
+    return out
+
+
+def run_tokenizer_decodes(arm):
+    """`decode_token_type` of every field, `compute_ticks` and both `compute_position_shifts` modes on random pieces (default_rng(5))
+    with one or several (compound) metres, for the SPMuple and SPMuple2 families; `arm(spm2)` -> the object whose methods run."""
+    rng = np.random.default_rng(5)
+    out = {}
+    for spm2 in (False, True):
+        tok = arm(spm2)
+        for trial in range(6):
+            piece = make_piece(int(rng.integers(5, 300)), int(rng.integers(10000)), metre_change=bool(trial % 2))
+            if trial >= 3:                                  # several metre changes, compound metres included
+                bars = piece[:, 0] - 4
+                piece[:, 6] = 4 + (bars // int(rng.integers(2, 6))) % 22
+            tag = f"spm{2 if spm2 else 1}/t{trial}"
+            for field in FIELDS:
+                out[f"{tag}/{field}"] = np.asarray(tok.decode_token_type(piece, field))
+            ticks = tok.compute_ticks(piece.copy(), 8, compute_beat_ticks=True)
+            for key in ("note_on", "bar", "beat"):
+                out[f"{tag}/ticks_{key}"] = np.asarray(ticks[key])
+            out[f"{tag}/metres"], out[f"{tag}/metre_ticks"] = np.asarray(ticks["time_sig"][0]), np.asarray(ticks["time_sig"][1])
+            on = np.sort(ticks["note_on"])
+            for mode in (True, False):
+                out[f"{tag}/shifts_{int(mode)}"] = np.asarray(tok.compute_position_shifts(on.copy(), onset_shift=mode))
+    return out
+
+
 # ----------------------------------------------------------------------------- encode_embeddings: a dataset that serves bar windows
 class _Scores(list):
     _name_to_idx = {"score0": 0}

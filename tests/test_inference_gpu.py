@@ -140,9 +140,6 @@ def test_render_performances_batches_whole_pieces():
         assert agree > 0.85, agree
 
 
-@pytest.mark.xfail(strict=False, reason="written after the round's GPU budget was spent: never run on a GPU by its author (the host logic is "
-                                        "pinned on CPU in tests/test_inference_host.py; the device path is the one the tests above use, "
-                                        "with more notes per call) -- expected to pass, reported as XPASS when it does")
 def test_lookahead_rendering_on_device_equals_chord_by_chord_rendering():
     """`lookahead_notes`: several chords per decoder call on the CUDA decoder must render what chord-by-chord calls render (greedy),
     with fewer calls."""

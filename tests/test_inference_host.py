@@ -19,6 +19,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "oracle"))
 
 import inference_cases as cases  # noqa: E402
+from tests import parity  # noqa: E402
 from scoreperformer_b200.inference import (ScorePerformerGenerator, SPMuple2IntermediateData, SPMuple2Messenger, SPMupleMessenger,  # noqa: E402
                                            TokenTables)
 from scoreperformer_b200.inference.token_tables import find_closest  # noqa: E402
@@ -187,13 +188,11 @@ def test_cut_caches_views_and_window_helpers():
 
 
 def _reference_root():
-    for cand in (os.path.join(ROOT, "baseline", "_ref"), "/root/reference"):
-        if os.path.isdir(os.path.join(cand, "scoreperformer", "inference")):
-            return cand
-    return None
+    root = parity.reference_root()
+    return root if root is not None and os.path.isdir(os.path.join(root, "scoreperformer", "inference")) else None
 
 
-@pytest.mark.skipif(_reference_root() is None, reason="needs the unmodified reference (baseline/_ref or /root/reference)")
+@pytest.mark.skipif(_reference_root() is None, reason="needs a copy of the original ScorePerformer project ($SPB200_REFERENCE_ROOT or baseline/_ref)")
 def test_loop_around_the_reference_model_matches_the_reference_loop():
     """Live, not from goldens: the UNMODIFIED reference model (default recipe, CPU fp32, cached `unmask_tokens`) rendered once by the
     reference's generator + messenger and once by this package's -- same windows, caches handed back and forth between the reference's
@@ -347,114 +346,93 @@ def test_tables_from_a_tokenizer_preset():
     assert messages.shape == (240, 4) and np.isfinite(messages).all() and np.all(np.diff(messages[:, 0]) >= 0)
 
 
-@pytest.mark.skipif(_reference_root() is None, reason="needs the unmodified reference (baseline/_ref or /root/reference)")
-def test_random_renderings_match_the_reference_loop_live():
-    """Beyond the four goldens: random pieces, contexts, window lengths, chord grouping, style deltas, cache use, tempo modes and
-    masked field sets, rendered live by the reference's generator + messenger and by this package's around the stand-in decoder --
-    every decoder call and every window must agree exactly."""
+def _package_arms():
+    """This package's side of the seeded random cases of oracle/inference_cases.py."""
+    def render(spm2, params):
+        return (ScorePerformerGenerator, SPMuple2Messenger if spm2 else SPMupleMessenger,
+                TokenTables(**cases.table_kwargs(**params), spmuple2=spm2), (Caches, Inter, Attn), SPMuple2IntermediateData)
+
+    def messenger(spm2, params):
+        return (SPMuple2Messenger if spm2 else SPMupleMessenger)(TokenTables(**cases.table_kwargs(**params), spmuple2=spm2))
+    return render, messenger, lambda spm2: TokenTables(**cases.table_kwargs())
+
+
+def _reference_arms():
     os.environ["SPB200_REFERENCE_ROOT"] = _reference_root()
     import gen_inference_golden as ref
-    rng = np.random.default_rng(2024)
-    names = []
-    for i in range(14):
-        params = [{}, dict(decode_recompute_tempos=False), dict(onset_tempos=True), dict(use_quantized_tempos=False, tempo_window=3.)][i % 4]
-        ignore = (0, 1, 2, 4, 6, 7, 8, 9) if i % 3 else (0, 1, 2, 4, 5, 6, 7, 8, 9)
-        gen_kw = dict(max_context_len=int(rng.choice([24, 40, 64, 512])), group_chord_notes=bool(rng.random() < 0.7),
-                      time_window_overflow=float(rng.choice([0., 0.1, 0.3])), disable_caches=bool(rng.random() < 0.2),
-                      delta=bool(rng.random() < 0.4), sort_messages=bool(rng.random() < 0.5))
-        name = f"fuzz{i}"
-        cases.SCENARIOS[name] = (dict(n_notes=int(rng.integers(40, 160)), seed=int(rng.integers(1000))), params, ignore, gen_kw,
-                                 float(rng.choice([0.25, 0.5, 1.0, 2.5])), "spm2")
-        names.append(name)
+
+    def render(spm2, params):
+        return (ref.ScorePerformerGenerator, ref.SPMuple2Messenger if spm2 else ref.SPMupleMessenger,
+                ref._ref_tokenizer(ref.SPMuple2 if spm2 else ref.SPMuple, **params), ref.REF_CACHES, ref.SPMuple2IntermediateData)
+
+    def messenger(spm2, params):
+        return (ref.SPMuple2Messenger if spm2 else ref.SPMupleMessenger)(ref._ref_tokenizer(ref.SPMuple2 if spm2 else ref.SPMuple, **params))
+    return render, messenger, lambda spm2: ref._ref_tokenizer(ref.SPMuple2 if spm2 else ref.SPMuple)
+
+
+def live_records(native=True):
+    """This package's record of the seeded random cases, as tests/golden/inference_live.npz stores it (oracle/gen_live_golden.py)."""
+    render, messenger, tokenizer = _package_arms()
+    old = os.environ.get("SPB_HOST_NATIVE")
+    os.environ["SPB_HOST_NATIVE"] = "1" if native else "0"
     try:
-        for j, name in enumerate(names):
-            params = cases.SCENARIOS[name][1]
-            spm2 = j % 5 != 4                               # every fifth case: the SPMuple family (tick-based messenger, no tempo state)
-            want = cases.run_scenario(name, ref.ScorePerformerGenerator, ref.SPMuple2Messenger if spm2 else ref.SPMupleMessenger,
-                                      ref._ref_tokenizer(ref.SPMuple2 if spm2 else ref.SPMuple, **params), ref.REF_CACHES,
-                                      ref.SPMuple2IntermediateData)
-            got = cases.run_scenario(name, ScorePerformerGenerator, SPMuple2Messenger if spm2 else SPMupleMessenger,
-                                     TokenTables(**cases.table_kwargs(**params), spmuple2=spm2), (Caches, Inter, Attn),
-                                     SPMuple2IntermediateData)
-            assert len(got[0]) == len(want[0]), (name, cases.SCENARIOS[name])
-            for i, (a, b) in enumerate(zip(got[0], want[0])):
-                for k in a:
-                    same(a[k], b[k], f"{name} {cases.SCENARIOS[name]} window {i} {k}")
-            for k in got[1]:
-                same(got[1][k], want[1][k], f"{name} final {k}")
+        return {"render": cases.run_fuzz_renderings(render), "messenger": cases.run_messenger_configurations(messenger),
+                "tokenizer": cases.run_tokenizer_decodes(tokenizer)}
     finally:
-        for name in names:
-            cases.SCENARIOS.pop(name, None)
+        if old is None:
+            os.environ.pop("SPB_HOST_NATIVE")
+        else:
+            os.environ["SPB_HOST_NATIVE"] = old
 
 
-@pytest.mark.skipif(_reference_root() is None, reason="needs the unmodified reference (baseline/_ref or /root/reference)")
-def test_random_messenger_configurations_match_the_reference_live():
-    """Random tempo / shift / deviation settings, metre changes and chunkings through the reference's messengers and this package's
-    (C recurrence and numpy statement): messages, tick messages and carried state identical."""
-    os.environ["SPB200_REFERENCE_ROOT"] = _reference_root()
-    import gen_inference_golden as ref
-    rng = np.random.default_rng(77)
-    for i in range(16):
-        spm2 = i % 2 == 0
-        params = dict(decode_recompute_tempos=bool(rng.random() < 0.6), onset_tempos=bool(rng.random() < 0.25),
-                      use_quantized_tempos=bool(rng.random() < 0.5), tempo_window=float(rng.choice([1., 4., 8., 1e6])),
-                      tempo_min_onsets=int(rng.choice([2, 8, 40])), tempo_min_onset_dist=float(rng.choice([0.1, 0.5, 2.])),
-                      bar_tempos=bool(rng.random() < 0.5), use_position_shifts=bool(rng.random() < 0.5),
-                      onset_position_shifts=bool(rng.random() < 0.5), rel_onset_dev=True, rel_perf_duration=bool(spm2 or rng.random() < 0.7))
-        if not spm2 and not params["rel_perf_duration"]:
-            continue                                       # absolute PerfDuration needs its own vocabulary column
-        ref_tok = ref._ref_tokenizer(ref.SPMuple2 if spm2 else ref.SPMuple, **params)
-        ref_m = (ref.SPMuple2Messenger if spm2 else ref.SPMupleMessenger)(ref_tok)
-        piece, cuts = cases.random_chunks(int(rng.integers(10000)), n_notes=int(rng.integers(30, 400)), metre_change=bool(rng.random() < 0.4))
-        runs = {}
-        for arm in ("reference", "native", "numpy"):
-            if arm == "reference":
-                m = ref_m
-            else:
-                os.environ["SPB_HOST_NATIVE"] = "1" if arm == "native" else "0"
-                m = (SPMuple2Messenger if spm2 else SPMupleMessenger)(TokenTables(**cases.table_kwargs(**params), spmuple2=spm2))
-            state, lo, out = None, 0, []
-            for hi in cuts:
-                if not spm2:
-                    out.append(m.tokens_to_messages(piece[lo:hi].copy(), intermediates=state, to_times=False, sort=True))
-                msgs, state = m.tokens_to_messages(piece[lo:hi].copy(), intermediates=state, return_intermediates=True,
-                                                   sort=bool(hi % 2))
-                out.append(msgs)
-                lo = hi
-            runs[arm] = (np.concatenate(out), np.asarray(state.tempos, dtype=np.float64),
-                         np.asarray(getattr(state, "onset_pairs", None) if spm2 else [[0.]], dtype=np.float64))
-        os.environ.pop("SPB_HOST_NATIVE", None)
-        for arm in ("native", "numpy"):
-            for a, b, what in zip(runs[arm], runs["reference"], ("messages", "tempo map", "onset pairs")):
-                same(a, b, f"case {i} ({'SPMuple2' if spm2 else 'SPMuple'}, {params}) {arm}: {what}")
+@pytest.fixture(scope="module")
+def live_golden():
+    """The seeded random cases as this package rendered them at the commit whose inference code the live tests last found identical
+    to the original project (oracle/gen_live_golden.py); a copy of the original, where supplied, is compared live as well."""
+    return np.load(os.path.join(GOLDEN, "inference_live.npz"))
 
 
-@pytest.mark.skipif(_reference_root() is None, reason="needs the unmodified reference (baseline/_ref or /root/reference)")
-def test_token_tables_decode_like_the_reference_tokenizer_live():
-    """Every field's `decode_token_type`, `compute_ticks` on random metre sequences and both `compute_position_shifts` modes, live
-    against the reference tokenizer's own methods (OctupleM / SPMuple) on the same tables."""
-    os.environ["SPB200_REFERENCE_ROOT"] = _reference_root()
-    import gen_inference_golden as ref
-    rng = np.random.default_rng(5)
-    tables = TokenTables(**cases.table_kwargs())
-    for base in (ref.SPMuple, ref.SPMuple2):
-        tok = ref._ref_tokenizer(base)
-        for trial in range(6):
-            piece = cases.make_piece(int(rng.integers(5, 300)), int(rng.integers(10000)), metre_change=bool(trial % 2))
-            if trial >= 3:                                  # several metre changes, compound metres included
-                bars = piece[:, 0] - 4
-                piece[:, 6] = 4 + (bars // int(rng.integers(2, 6))) % 22
-            for field in cases.FIELDS:
-                same(tables.decode_token_type(piece, field), tok.decode_token_type(piece, field), f"{base.__name__} {field}")
-            want, got = tok.compute_ticks(piece.copy(), 8, compute_beat_ticks=True), tables.compute_ticks(piece.copy(), 8, compute_beat_ticks=True)
-            for key in ("note_on", "bar", "beat"):
-                same(got[key], want[key], f"{base.__name__} ticks {key} (trial {trial})")
-            same(got["time_sig"][0], want["time_sig"][0], "metres")
-            same(got["time_sig"][1], want["time_sig"][1], "metre ticks")
-            on = np.sort(want["note_on"])
-            for mode in (True, False):
-                same(tables.compute_position_shifts(on.copy(), onset_shift=mode), tok.compute_position_shifts(on.copy(), onset_shift=mode),
-                     f"position shifts onset_shift={mode}")
+@pytest.fixture(scope="module")
+def live_got():
+    return live_records(native=True)
+
+
+def _same_record(got, g, part, what):
+    want = {k[len(part) + 1:]: g[k] for k in g.files if k.startswith(part + "/")}
+    assert sorted(got) == sorted(want), f"{what}: keys differ"
+    for k in got:
+        same(got[k], want[k], f"{what} {k}")
+
+
+def test_random_renderings_match_the_reference_loop_live(live_golden, live_got):
+    """Beyond the four scenario goldens: 14 random pieces, contexts, window lengths, chord grouping, style deltas, cache use, tempo
+    modes and masked field sets around the stand-in decoder -- every decoder call and every window equal to the stored record, and
+    to the original project's generator + messenger live where a copy is supplied."""
+    _same_record(live_got["render"], live_golden, "render", "stored")
+    if _reference_root() is not None:
+        _same_record(live_got["render"], {f"render/{k}": v for k, v in cases.run_fuzz_renderings(_reference_arms()[0]).items()},
+                     "render", "original")
+
+
+def test_random_messenger_configurations_match_the_reference_live(live_golden, live_got):
+    """Random tempo / shift / deviation settings, metre changes and chunkings through this package's messengers (C recurrence and
+    numpy statement): messages, tick messages and carried state equal to the stored record, and to the original's messengers live
+    where a copy is supplied."""
+    _same_record(live_got["messenger"], live_golden, "messenger", "stored, C recurrence")
+    _same_record(live_records(native=False)["messenger"], live_golden, "messenger", "stored, numpy statement")
+    if _reference_root() is not None:
+        _same_record(live_got["messenger"], {f"messenger/{k}": v for k, v in cases.run_messenger_configurations(_reference_arms()[1]).items()},
+                     "messenger", "original")
+
+
+def test_token_tables_decode_like_the_reference_tokenizer_live(live_golden, live_got):
+    """Every field's `decode_token_type`, `compute_ticks` on random metre sequences and both `compute_position_shifts` modes of
+    TokenTables equal to the stored record, and to the original tokenizer's own methods (SPMuple / SPMuple2) live where a copy is
+    supplied."""
+    _same_record(live_got["tokenizer"], live_golden, "tokenizer", "stored")
+    if _reference_root() is not None:
+        _same_record(live_got["tokenizer"], {f"tokenizer/{k}": v for k, v in cases.run_tokenizer_decodes(_reference_arms()[2]).items()},
+                     "tokenizer", "original")
 
 
 def test_host_abi_from_a_c_program(tmp_path):

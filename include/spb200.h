@@ -96,7 +96,7 @@ int spb_decode_stack_step(const float* x_in, const float* style, int S, const vo
 int spb_gather_at_pos(const void* const* srcs, void* const* dsts, const int* row_bytes, const int* shifts, int n, const long long* pos_dev,
                       int B, int T, spb_stream_t stream);
 
-/* Tied heads of the rendered fields + sampling in one launch (modules/sampling.py:28-59, wrappers.py:358-397): per listed field
+/* Tied heads of the rendered fields + sampling in one launch (modules/sampling.py:12-59, wrappers.py:358-397): per listed field
  * (host int arrays: field index, first table row, vocabulary <= 256, top-k <= 32; k = 1 is greedy) logits = e_f . table_f^T stay in
  * registers, tokens [0, n_banned) are never emitted, and the drawn token is written to tokens[b, *pos_dev + 1, field] (int64 [B,T,F]).
  * advance (uint32 [2], may be NULL; [0] must be zero): the last CTA to finish does *pos_dev += 1 and clears advance[0] and advance[1]
@@ -104,6 +104,17 @@ int spb_gather_at_pos(const void* const* srcs, void* const* dsts, const int* row
 int spb_sample_fields(const void* e, int ld_e, const void* table, const int* fields, const int* offsets, const int* vocab, const int* topk,
                       int n_fields, int n_banned, float temperature, uint64_t seed, const long long* pos_dev, long long* tokens, int B,
                       int T, int F, unsigned* advance, spb_stream_t stream);
+/* spb_sample_fields with the other logit filters of modules/sampling.py and per-field bans (wrappers.py:358-397 filter_key_ids).  Per
+ * listed field, host arrays (each may be NULL = off for every field): top_p[i] >= 0 samples from the nucleus of that threshold (0 keeps
+ * the arg-max only; < 0 = off); top_a_ratio[i] > 0 keeps the tokens whose probability is at least max_prob^top_a_pow[i] * top_a_ratio[i]
+ * (max_prob of the score's own row; <= 0 = off); a field with neither samples top-k with topk[i].  At most one filter per field, finite
+ * parameters.  ban_bits[8 i .. 8 i + 7] is a 256-bit set of tokens field i never emits, applied together with [0, n_banned) before
+ * the filter (at least one token must remain).  Both filters see the softmax at temperature 1; the kept tokens are drawn from at
+ * `temperature`.  With every filter off the draws equal spb_sample_fields'. */
+int spb_sample_fields_filtered(const void* e, int ld_e, const void* table, const int* fields, const int* offsets, const int* vocab,
+                               const int* topk, int n_fields, int n_banned, float temperature, uint64_t seed, const long long* pos_dev,
+                               long long* tokens, int B, int T, int F, unsigned* advance, const float* top_p, const float* top_a_pow,
+                               const float* top_a_ratio, const uint32_t* ban_bits, spb_stream_t stream);
 
 /* Device side of the collator (data/collators/performance.py:239-255 MixedLM mask_sequence, score_performance.py:186-234): expands a
  * packed batch -- uint16 tokens, int32 segment ids [3, n] (bars | beats | onsets), uint8 directions, int32 lengths -- into the int64

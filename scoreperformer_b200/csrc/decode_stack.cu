@@ -28,6 +28,8 @@
 // a rendering is bit-reproducible.
 // Algorithmic HBM/L2 bytes per note-step: B * pos * 4 layers * 256 B of KV cache (the roofline term, SURVEY 8(d)) + 7.6 MB of
 // weights out of L2.
+#include <cmath>
+
 #include "common.cuh"
 
 namespace {
@@ -914,9 +916,13 @@ extern "C" int spb_gather_at_pos(const void* const* srcs, void* const* dsts, con
 // warp per field: logits = e_f . table_f^T stay in registers (V <= 256: up to 8 per lane), the k largest are peeled off by k
 // warp-wide arg-max rounds (k = 1 is greedy decoding: the lowest index wins ties, like torch.argmax), the draw uses a counter
 // based hash of (seed, position, score, field), and the token goes straight into tokens[b, pos + 1, field].
+// A field may instead carry top-p (sampling.py:12-18) or top-a (sampling.py:29-32): its logits are bitonic-sorted across the warp
+// (descending, the lowest index first among equal values), the filter keeps a prefix of that order by the temperature-1 softmax,
+// and the draw runs over the kept prefix.  Per-field token bans (a 256-bit mask) are applied before any filter.
 namespace {
 
 constexpr int SF_MAX_FIELDS = 8;
+constexpr int SF_TOPK = 0, SF_TOPP = 1, SF_TOPA = 2;        // filter of a field
 
 struct SampleParams {
     const __nv_bfloat16* e;       // [B, ld_e] normalised head projection (all fields)
@@ -924,6 +930,9 @@ struct SampleParams {
     const __nv_bfloat16* table;   // [sum V, 128]
     int n_fields;
     int field[SF_MAX_FIELDS], offset[SF_MAX_FIELDS], V[SF_MAX_FIELDS], k[SF_MAX_FIELDS];
+    int filter[SF_MAX_FIELDS];    // SF_TOPK (k above), SF_TOPP (thres in fa) or SF_TOPA (min_p_pow in fa, min_p_ratio in fb)
+    float fa[SF_MAX_FIELDS], fb[SF_MAX_FIELDS];
+    uint32_t ban[SF_MAX_FIELDS][8];   // token v of field w is never emitted if bit v of ban[w] is set
     int n_banned;                 // tokens [0, n_banned) are never emitted
     float inv_temperature;
     uint64_t seed;
@@ -933,59 +942,11 @@ struct SampleParams {
     unsigned* advance;            // optional [2]: [0] = CTA counter (zero between launches), [1] = word to clear (the stack kernel's barrier)
 };
 
-__global__ void __launch_bounds__(32 * SF_MAX_FIELDS)
-sample_fields_kernel(SampleParams p) {
-    const int b = blockIdx.x, w = threadIdx.x >> 5, lane = threadIdx.x & 31;      // the block has exactly n_fields warps
-    const int f = p.field[w], V = p.V[w], k = p.k[w];
-    const long long pos = *p.pos_dev;
-    // logits of 32 vocabulary rows at a time: every lane multiplies ITS four dims of e with the same four dims of each row (one
-    // coalesced 256-byte row per load instruction; a lane reading whole rows costs 32 L1 wavefronts per instruction), then a
-    // transposing butterfly (31 shuffles) leaves the complete dot product of row 32 i + L in lane L
-    float e4[4];
-    {
-        const uint2 u = *reinterpret_cast<const uint2*>(p.e + (size_t)b * p.ld_e + f * 128 + lane * 4);
-        const float2 a = unpack_bf16x2(u.x), c = unpack_bf16x2(u.y);
-        e4[0] = a.x; e4[1] = a.y; e4[2] = c.x; e4[3] = c.y;
-    }
-    const __nv_bfloat16* tbase = p.table + (size_t)p.offset[w] * 128 + lane * 4;
-    __shared__ float s_lg[SF_MAX_FIELDS][256];
-    uint2 un[32];                                            // the rows of the next group are in flight while this one is reduced
-#pragma unroll
-    for (int r = 0; r < 32; ++r) un[r] = r < V ? __ldg(reinterpret_cast<const uint2*>(tbase + (size_t)r * 128)) : make_uint2(0u, 0u);
-#pragma unroll 1                                             // one copy of the 32-row body: the kernel is short, its code should be too
-    for (int i = 0; i < 8; ++i) {
-        s_lg[w][lane + 32 * i] = -INFINITY;
-        if (32 * i >= V) continue;                           // warp-uniform
-        float x[32];
-#pragma unroll
-        for (int r = 0; r < 32; ++r) {
-            const float2 a = unpack_bf16x2(un[r].x), c = unpack_bf16x2(un[r].y);
-            x[r] = e4[0] * a.x + e4[1] * a.y + e4[2] * c.x + e4[3] * c.y;
-        }
-        if (32 * (i + 1) < V) {
-#pragma unroll
-            for (int r = 0; r < 32; ++r) {
-                const int v = 32 * (i + 1) + r;
-                un[r] = v < V ? __ldg(reinterpret_cast<const uint2*>(tbase + (size_t)v * 128)) : make_uint2(0u, 0u);
-            }
-        }
-#pragma unroll
-        for (int s_ = 16; s_ >= 1; s_ >>= 1) {
-            const bool upper = (lane & s_) != 0;
-#pragma unroll
-            for (int r = 0; r < s_; ++r) {
-                const float send = upper ? x[r] : x[r + s_];
-                const float keep = upper ? x[r + s_] : x[r];
-                x[r] = keep + __shfl_xor_sync(0xffffffffu, send, s_);
-            }
-        }
-        const int v = lane + 32 * i;
-        if (v < V && v >= p.n_banned) s_lg[w][v] = x[0];
-    }
-    __syncwarp();
+// top-k (k = 1: greedy) over the logits of one field, lg_row = its 256 logits in shared memory (-inf: banned / beyond V)
+__device__ __forceinline__ int sample_topk(const SampleParams& p, const float* lg_row, int k, int b, int w, int lane, long long pos) {
     float lg[8];
 #pragma unroll
-    for (int i = 0; i < 8; ++i) lg[i] = s_lg[w][lane + 32 * i];
+    for (int i = 0; i < 8; ++i) lg[i] = lg_row[lane + 32 * i];
     // k rounds of warp arg-max: round t leaves its winner (value, token) in lane t
     float top_val = -INFINITY;
     int top_idx = 0;
@@ -1026,6 +987,160 @@ sample_fields_kernel(SampleParams p) {
         const int pick = ge != 0 ? __ffs(ge) - 1 : k - 1;
         token = __shfl_sync(0xffffffffu, top_idx, pick);
     }
+    return token;
+}
+
+// top-p / top-a over the logits of one field.  The 256 (logit, token) pairs are sorted across the warp -- descending, the lowest
+// token first among equal logits (the greedy rule) -- by a bitonic network, lane L ending with ranks 8L .. 8L+7 (strides < 8 are
+// exchanges inside a lane, the others shuffles).  The temperature-1 softmax q_r / Z of the sorted logits decides which prefix of
+// ranks is kept, rank 0 always:
+//   top-p (sampling.py:12-18): rank r >= 1 is kept iff q_0 + ... + q_{r-1} <= thres Z  (the reference's `cum > thres` shifted by one);
+//   top-a (sampling.py:29-32): rank r is kept iff q_r / Z >= (1 / Z)^min_p_pow min_p_ratio  (1 / Z = the largest probability).
+// The kept ranks are drawn from as in top-k: softmax at the temperature, inverse cdf with the same counter hash.
+__device__ __forceinline__ int sample_sorted(const SampleParams& p, const float* lg_row, int b, int w, int lane, long long pos) {
+    float val[8];
+    int idx[8];
+    {
+        const float4 a = *reinterpret_cast<const float4*>(lg_row + 8 * lane);
+        const float4 c = *reinterpret_cast<const float4*>(lg_row + 8 * lane + 4);
+        val[0] = a.x; val[1] = a.y; val[2] = a.z; val[3] = a.w; val[4] = c.x; val[5] = c.y; val[6] = c.z; val[7] = c.w;
+    }
+#pragma unroll
+    for (int i = 0; i < 8; ++i) idx[i] = 8 * lane + i;
+    // x comes before y in the sorted order (token indices are unique: a strict total order)
+    auto before = [](float xv, int xi, float yv, int yi) { return xv > yv || (xv == yv && xi < yi); };
+#pragma unroll
+    for (int kk = 2; kk <= 256; kk <<= 1) {
+#pragma unroll
+        for (int j = kk >> 1; j > 0; j >>= 1) {
+            if (j >= 8) {
+                const int lj = j >> 3;
+                const bool lower = (lane & lj) == 0;
+#pragma unroll
+                for (int i = 0; i < 8; ++i) {
+                    // the lower element of the pair takes the one that comes first when (rank & kk) == 0, else the one after
+                    const bool take_first = lower == (((8 * lane + i) & kk) == 0);
+                    const float ov = __shfl_xor_sync(0xffffffffu, val[i], lj);
+                    const int oi = __shfl_xor_sync(0xffffffffu, idx[i], lj);
+                    if (before(ov, oi, val[i], idx[i]) == take_first) { val[i] = ov; idx[i] = oi; }
+                }
+            } else {
+#pragma unroll
+                for (int i = 0; i < 8; ++i) {
+                    if (i & j) continue;
+                    const bool first_low = ((8 * lane + i) & kk) == 0;
+                    if (before(val[i | j], idx[i | j], val[i], idx[i]) == first_low) {
+                        const float tv = val[i]; val[i] = val[i | j]; val[i | j] = tv;
+                        const int ti = idx[i]; idx[i] = idx[i | j]; idx[i | j] = ti;
+                    }
+                }
+            }
+        }
+    }
+    // temperature-1 weights q = exp(logit - max) and the mass of the ranks before this lane's first (warp scan)
+    const float m = __shfl_sync(0xffffffffu, val[0], 0);
+    float q[8], s = 0.f;
+#pragma unroll
+    for (int i = 0; i < 8; ++i) { q[i] = __expf(val[i] - m); s += q[i]; }       // banned / beyond V: exp(-inf) = 0
+    float incl = s;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const float up = __shfl_up_sync(0xffffffffu, incl, o);
+        if (lane >= o) incl += up;
+    }
+    const float Z = __shfl_sync(0xffffffffu, incl, 31);
+    float cum = __shfl_up_sync(0xffffffffu, incl, 1);
+    if (lane == 0) cum = 0.f;
+    const bool top_p = p.filter[w] == SF_TOPP;
+    const float lim = top_p ? p.fa[w] * Z : __powf(1.f / Z, p.fa[w]) * p.fb[w] * Z;
+    float wt[8], ws = 0.f;
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+        const bool keep = (lane == 0 && i == 0) || (top_p ? cum <= lim : q[i] >= lim);
+        cum += q[i];
+        wt[i] = keep ? __expf((val[i] - m) * p.inv_temperature) : 0.f;
+        ws += wt[i];
+    }
+    // softmax of the kept ranks at the temperature, one draw by inverse cdf: the lane whose running sum passes u, then its rank
+    float wincl = ws;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const float up = __shfl_up_sync(0xffffffffu, wincl, o);
+        if (lane >= o) wincl += up;
+    }
+    const float total = __shfl_sync(0xffffffffu, wincl, 31);
+    float acc = __shfl_up_sync(0xffffffffu, wincl, 1);
+    if (lane == 0) acc = 0.f;
+    const uint32_t r = spb_hash32(p.seed + (uint64_t)pos * 0x9E3779B97F4A7C15ull, (uint64_t)b * SF_MAX_FIELDS + (uint64_t)w);
+    const float u = (float)(r >> 8) * (1.f / 16777216.f) * total;
+    const unsigned hit = __ballot_sync(0xffffffffu, ws > 0.f && wincl > u);
+    const unsigned nonzero = __ballot_sync(0xffffffffu, ws > 0.f);          // holds lane 0: rank 0 is always kept
+    const int src = hit != 0u ? __ffs(hit) - 1 : 31 - __clz(nonzero);
+    int token = idx[0];
+    bool found = false;
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+        if (wt[i] > 0.f && !found) {               // the last kept rank of the lane if rounding leaves u above its running sum
+            token = idx[i];
+            acc += wt[i];
+            found = acc > u;
+        }
+    }
+    return __shfl_sync(0xffffffffu, token, src);
+}
+
+__global__ void __launch_bounds__(32 * SF_MAX_FIELDS)
+sample_fields_kernel(SampleParams p) {
+    const int b = blockIdx.x, w = threadIdx.x >> 5, lane = threadIdx.x & 31;      // the block has exactly n_fields warps
+    const int f = p.field[w], V = p.V[w], k = p.k[w];
+    const long long pos = *p.pos_dev;
+    // logits of 32 vocabulary rows at a time: every lane multiplies ITS four dims of e with the same four dims of each row (one
+    // coalesced 256-byte row per load instruction; a lane reading whole rows costs 32 L1 wavefronts per instruction), then a
+    // transposing butterfly (31 shuffles) leaves the complete dot product of row 32 i + L in lane L
+    float e4[4];
+    {
+        const uint2 u = *reinterpret_cast<const uint2*>(p.e + (size_t)b * p.ld_e + f * 128 + lane * 4);
+        const float2 a = unpack_bf16x2(u.x), c = unpack_bf16x2(u.y);
+        e4[0] = a.x; e4[1] = a.y; e4[2] = c.x; e4[3] = c.y;
+    }
+    const __nv_bfloat16* tbase = p.table + (size_t)p.offset[w] * 128 + lane * 4;
+    __shared__ __align__(16) float s_lg[SF_MAX_FIELDS][256];
+    uint2 un[32];                                            // the rows of the next group are in flight while this one is reduced
+#pragma unroll
+    for (int r = 0; r < 32; ++r) un[r] = r < V ? __ldg(reinterpret_cast<const uint2*>(tbase + (size_t)r * 128)) : make_uint2(0u, 0u);
+#pragma unroll 1                                             // one copy of the 32-row body: the kernel is short, its code should be too
+    for (int i = 0; i < 8; ++i) {
+        s_lg[w][lane + 32 * i] = -INFINITY;
+        if (32 * i >= V) continue;                           // warp-uniform
+        float x[32];
+#pragma unroll
+        for (int r = 0; r < 32; ++r) {
+            const float2 a = unpack_bf16x2(un[r].x), c = unpack_bf16x2(un[r].y);
+            x[r] = e4[0] * a.x + e4[1] * a.y + e4[2] * c.x + e4[3] * c.y;
+        }
+        if (32 * (i + 1) < V) {
+#pragma unroll
+            for (int r = 0; r < 32; ++r) {
+                const int v = 32 * (i + 1) + r;
+                un[r] = v < V ? __ldg(reinterpret_cast<const uint2*>(tbase + (size_t)v * 128)) : make_uint2(0u, 0u);
+            }
+        }
+#pragma unroll
+        for (int s_ = 16; s_ >= 1; s_ >>= 1) {
+            const bool upper = (lane & s_) != 0;
+#pragma unroll
+            for (int r = 0; r < s_; ++r) {
+                const float send = upper ? x[r] : x[r + s_];
+                const float keep = upper ? x[r + s_] : x[r];
+                x[r] = keep + __shfl_xor_sync(0xffffffffu, send, s_);
+            }
+        }
+        const int v = lane + 32 * i;
+        if (v < V && v >= p.n_banned && ((p.ban[w][i] >> lane) & 1u) == 0u) s_lg[w][v] = x[0];
+    }
+    __syncwarp();
+    const int token = p.filter[w] == SF_TOPK ? sample_topk(p, s_lg[w], k, b, w, lane, pos)
+                                             : sample_sorted(p, s_lg[w], b, w, lane, pos);
     if (lane == 0 && pos + 1 < p.T) p.tokens[((size_t)b * p.T + (size_t)(pos + 1)) * p.F + f] = token;
     if (p.advance != nullptr) {
         // the last CTA to finish ends the note-step: position += 1 and the decode-stack kernel's grid-barrier word back to zero
@@ -1047,27 +1162,71 @@ sample_fields_kernel(SampleParams p) {
 
 }  // namespace
 
-// e bf16 [B, ld_e] (LayerNorm'ed head projection, 128 columns per field), table bf16 [sum V, 128]; for each of the n_fields listed
-// fields (field index, first table row, vocabulary, k of the top-k filter; k = 1: greedy) one token is written to
-// tokens[b, *pos_dev + 1, field] (int64 [B, T, F]).  V <= 256, k <= 32, at most 8 fields.
-extern "C" int spb_sample_fields(const void* e, int ld_e, const void* table, const int* fields, const int* offsets, const int* vocab,
-                                 const int* topk, int n_fields, int n_banned, float temperature, uint64_t seed, const long long* pos_dev,
-                                 long long* tokens, int B, int T, int F, unsigned* advance, cudaStream_t stream) {
+namespace {
+
+// Both entry points: the filter arrays may be NULL (every field top-k, no per-field bans).
+int launch_sample_fields(const char* name, const void* e, int ld_e, const void* table, const int* fields, const int* offsets,
+                         const int* vocab, const int* topk, int n_fields, int n_banned, float temperature, uint64_t seed,
+                         const long long* pos_dev, long long* tokens, int B, int T, int F, unsigned* advance, const float* top_p,
+                         const float* top_a_pow, const float* top_a_ratio, const uint32_t* ban_bits, cudaStream_t stream) {
     if (B <= 0 || n_fields <= 0) return SPB_OK;
-    SPB_CHECK_ARG(e && table && fields && offsets && vocab && topk && pos_dev && tokens, "spb_sample_fields: null pointer");
-    SPB_CHECK_ARG(n_fields <= SF_MAX_FIELDS && ld_e % 4 == 0 && temperature > 0.f, "spb_sample_fields: at most %d fields, ld_e %% 4 == 0, temperature > 0", SF_MAX_FIELDS);
+    SPB_CHECK_ARG(e && table && fields && offsets && vocab && topk && pos_dev && tokens, "%s: null pointer", name);
+    SPB_CHECK_ARG(n_fields <= SF_MAX_FIELDS && ld_e % 4 == 0 && temperature > 0.f, "%s: at most %d fields, ld_e %% 4 == 0, temperature > 0", name, SF_MAX_FIELDS);
+    SPB_CHECK_ARG((top_a_pow == nullptr) == (top_a_ratio == nullptr), "%s: top_a_pow and top_a_ratio go together", name);
     SampleParams p;
     p.e = reinterpret_cast<const __nv_bfloat16*>(e); p.ld_e = ld_e;
     p.table = reinterpret_cast<const __nv_bfloat16*>(table);
     p.n_fields = n_fields;
     for (int i = 0; i < n_fields; ++i) {
         SPB_CHECK_ARG(vocab[i] >= 1 && vocab[i] <= 256 && topk[i] >= 1 && topk[i] <= 32 && fields[i] >= 0 && fields[i] < F,
-                      "spb_sample_fields: field %d needs V <= 256 and 1 <= k <= 32 (V %d, k %d)", fields[i], vocab[i], topk[i]);
+                      "%s: field %d needs V <= 256 and 1 <= k <= 32 (V %d, k %d)", name, fields[i], vocab[i], topk[i]);
         p.field[i] = fields[i]; p.offset[i] = offsets[i]; p.V[i] = vocab[i]; p.k[i] = topk[i] < vocab[i] ? topk[i] : vocab[i];
+        p.filter[i] = SF_TOPK; p.fa[i] = 0.f; p.fb[i] = 0.f;
+        const bool want_p = top_p != nullptr && top_p[i] >= 0.f, want_a = top_a_ratio != nullptr && top_a_ratio[i] > 0.f;
+        SPB_CHECK_ARG(top_p == nullptr || std::isfinite(top_p[i]), "%s: field %d: top_p must be finite (< 0 = off)", name, fields[i]);
+        SPB_CHECK_ARG(top_a_pow == nullptr || (std::isfinite(top_a_pow[i]) && std::isfinite(top_a_ratio[i])),
+                      "%s: field %d: top-a parameters must be finite (ratio <= 0 = off)", name, fields[i]);
+        SPB_CHECK_ARG(!(want_p && want_a), "%s: field %d: at most one of top-p and top-a", name, fields[i]);
+        if (want_p) { p.filter[i] = SF_TOPP; p.fa[i] = top_p[i]; }
+        if (want_a) { p.filter[i] = SF_TOPA; p.fa[i] = top_a_pow[i]; p.fb[i] = top_a_ratio[i]; }
+        int left = 0;                                        // tokens the field may still emit
+        for (int wd = 0; wd < 8; ++wd) {
+            p.ban[i][wd] = ban_bits != nullptr ? ban_bits[8 * i + wd] : 0u;
+            for (int bit = 0; bit < 32; ++bit) {
+                const int v = 32 * wd + bit;
+                left += v >= n_banned && v < vocab[i] && ((p.ban[i][wd] >> bit) & 1u) == 0u;
+            }
+        }
+        SPB_CHECK_ARG(ban_bits == nullptr || left > 0, "%s: field %d: every token is banned", name, fields[i]);
     }
     p.n_banned = n_banned; p.inv_temperature = 1.f / temperature; p.seed = seed; p.pos_dev = pos_dev;
     p.tokens = tokens; p.T = T; p.F = F; p.advance = advance;
     sample_fields_kernel<<<B, 32 * n_fields, 0, stream>>>(p);
     SPB_CHECK_LAUNCH();
     return SPB_OK;
+}
+
+}  // namespace
+
+// e bf16 [B, ld_e] (LayerNorm'ed head projection, 128 columns per field), table bf16 [sum V, 128]; for each of the n_fields listed
+// fields (field index, first table row, vocabulary, k of the top-k filter; k = 1: greedy) one token is written to
+// tokens[b, *pos_dev + 1, field] (int64 [B, T, F]).  V <= 256, k <= 32, at most 8 fields.
+extern "C" int spb_sample_fields(const void* e, int ld_e, const void* table, const int* fields, const int* offsets, const int* vocab,
+                                 const int* topk, int n_fields, int n_banned, float temperature, uint64_t seed, const long long* pos_dev,
+                                 long long* tokens, int B, int T, int F, unsigned* advance, cudaStream_t stream) {
+    return launch_sample_fields("spb_sample_fields", e, ld_e, table, fields, offsets, vocab, topk, n_fields, n_banned, temperature, seed,
+                                pos_dev, tokens, B, T, F, advance, nullptr, nullptr, nullptr, nullptr, stream);
+}
+
+// spb_sample_fields with per-field filters (host arrays, each may be NULL = off for every field): top_p[i] >= 0 selects top-p with
+// that threshold (0 keeps the arg-max only), top_a_ratio[i] > 0 selects top-a with (top_a_pow[i], top_a_ratio[i]); a field with
+// neither samples top-k with topk[i].  ban_bits[8 i .. 8 i + 7] (uint32) is a 256-bit set of tokens field i never emits, applied
+// with [0, n_banned) before the filter.
+extern "C" int spb_sample_fields_filtered(const void* e, int ld_e, const void* table, const int* fields, const int* offsets, const int* vocab,
+                                          const int* topk, int n_fields, int n_banned, float temperature, uint64_t seed,
+                                          const long long* pos_dev, long long* tokens, int B, int T, int F, unsigned* advance,
+                                          const float* top_p, const float* top_a_pow, const float* top_a_ratio, const uint32_t* ban_bits,
+                                          cudaStream_t stream) {
+    return launch_sample_fields("spb_sample_fields_filtered", e, ld_e, table, fields, offsets, vocab, topk, n_fields, n_banned, temperature,
+                                seed, pos_dev, tokens, B, T, F, advance, top_p, top_a_pow, top_a_ratio, ban_bits, stream);
 }

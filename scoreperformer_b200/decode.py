@@ -13,7 +13,7 @@ Two entry points over the same kernels:
 from __future__ import annotations
 
 import math
-from typing import Callable, Dict, List, Optional, Sequence
+from typing import Callable, Dict, List, Optional, Sequence, Tuple, Union
 
 import torch
 from torch import Tensor
@@ -119,23 +119,57 @@ def cached_stack_step(tr, x: Tensor, mask: Optional[Tensor], style: Optional[Ten
 
 @torch.no_grad()
 def render_batch(model, perf: Tensor, masked_perf: Tensor, score_hidden: Tensor, style: Tensor, mask: Optional[Tensor] = None,
-                 fields: Sequence[int] = (3, 5, 10, 11), temperature: float = 1.0, top_k: Optional[int] = 1,
-                 generator: Optional[torch.Generator] = None, teacher: Optional[Tensor] = None, use_graph: bool = True) -> Tensor:
+                 fields: Sequence[int] = (3, 5, 10, 11), temperature: float = 1.0, top_k: Union[int, Sequence[int], None] = 1,
+                 generator: Optional[torch.Generator] = None, teacher: Optional[Tensor] = None, use_graph: bool = True,
+                 top_p: Optional[float] = None, top_a: Optional[Tuple[float, float]] = None,
+                 banned_tokens: Optional[Dict[int, Sequence[int]]] = None) -> Tensor:
     """`render_decoder` on the performance decoder of a ScorePerformer model."""
     return render_decoder(model.perf_decoder.model, perf, masked_perf, score_hidden, style, mask=mask, fields=fields,
-                          temperature=temperature, top_k=top_k, generator=generator, teacher=teacher, use_graph=use_graph)
+                          temperature=temperature, top_k=top_k, generator=generator, teacher=teacher, use_graph=use_graph,
+                          top_p=top_p, top_a=top_a, banned_tokens=banned_tokens)
+
+
+def _check_filters(top_k, top_p, top_a, banned_tokens, fields: Sequence[int], sizes: Sequence[int], n_special: int = 2):
+    """Validate the sampling request of `render_decoder`; returns the per-field lists of banned ids (empty lists: none)."""
+    if top_p is not None and top_a is not None:
+        raise ValueError("top_p and top_a are two logit filters: pass at most one")
+    if (top_p is not None or top_a is not None) and top_k not in (None, 1):
+        raise ValueError(f"top_k={top_k!r} cannot be combined with top_p / top_a: pass top_k=None (or 1)")
+    if top_p is not None and not (math.isfinite(float(top_p)) and float(top_p) >= 0.0):
+        raise ValueError(f"top_p must be a finite threshold >= 0, got {top_p!r}")
+    if top_a is not None:
+        if len(top_a) != 2 or not all(math.isfinite(float(x)) for x in top_a) or float(top_a[1]) <= 0.0:
+            raise ValueError(f"top_a must be a finite (min_p_pow, min_p_ratio) pair with min_p_ratio > 0, got {top_a!r}")
+    bans = [[] for _ in fields]
+    for f, ids in (banned_tokens or {}).items():
+        if f not in fields:
+            raise ValueError(f"banned_tokens names field {f}, which is not rendered (fields {list(fields)})")
+        ids = sorted({int(v) for v in ids})
+        bad = [v for v in ids if not 0 <= v < sizes[f]]
+        if bad:
+            raise ValueError(f"banned_tokens of field {f}: ids {bad} are outside its vocabulary of {sizes[f]}")
+        if len(set(ids) | set(range(n_special))) >= sizes[f]:
+            raise ValueError(f"banned_tokens of field {f} leave no token to emit")
+        bans[list(fields).index(f)] = ids
+    return bans
 
 
 @torch.no_grad()
 def render_decoder(dec, perf: Tensor, masked_perf: Tensor, score_hidden: Tensor, style: Tensor, mask: Optional[Tensor] = None,
-                   fields: Sequence[int] = (3, 5, 10, 11), temperature: float = 1.0, top_k: Optional[int] = 1,
+                   fields: Sequence[int] = (3, 5, 10, 11), temperature: float = 1.0, top_k: Union[int, Sequence[int], None] = 1,
                    generator: Optional[torch.Generator] = None, teacher: Optional[Tensor] = None, use_graph: bool = True,
-                   start: int = 0, kv_init: Optional[Sequence[Tensor]] = None, return_kv: bool = False):
+                   start: int = 0, kv_init: Optional[Sequence[Tensor]] = None, return_kv: bool = False, top_p: Optional[float] = None,
+                   top_a: Optional[Tuple[float, float]] = None, banned_tokens: Optional[Dict[int, Sequence[int]]] = None):
     """Fill `fields` of every note >= 1 of `perf` [B, T, F], note by note, for all B scores in lockstep.
 
     perf / masked_perf: int64 [B, T, F]; score_hidden fp32 [B, T, D]; style fp32 [B, T, S]; mask bool [B, T].
     `top_k=1` is greedy (the parity mode, `filter_kwargs={'k': 1}` in the reference); larger k samples from the top-k
-    softmax at `temperature`; `top_k=None` uses the reference default ceil(0.1 * V).
+    softmax at `temperature`; `top_k=None` uses the reference default ceil(0.1 * V); a sequence gives one k per field.
+    `top_p` (nucleus threshold, modules/sampling.py `top_p`; 0 keeps the arg-max only) or `top_a` ((min_p_pow, min_p_ratio),
+    `top_a`) replaces top-k -- then `top_k` must be None or 1.  Both filters see the softmax at temperature 1 of each score's own
+    logits (the reference's `top_a` takes its maximum probability over the whole batch it is handed; here it is per score, which
+    is the same for one score); the kept tokens are drawn from at `temperature`.  `banned_tokens` maps a field index to token ids
+    that field never emits (the reference's `filter_key_ids`), applied with the PAD / MASK ban before the filter.
     `teacher` [B, T, F] (optional) is fed as the already-rendered prefix instead of the model's own samples (teacher forcing,
     used by the parity tests to compare every step independently); the returned tensor still holds the model's predictions.
     `use_graph`: capture one note-step in a CUDA graph and replay it (positions are device-side); sampling with a custom
@@ -144,13 +178,15 @@ def render_decoder(dec, perf: Tensor, masked_perf: Tensor, score_hidden: Tensor,
     [B, s, 128] holds the keys | values of decoder positions < s for every layer, and only the positions s..T-2 run (notes s+1..T-1
     are rendered).  `return_kv` also returns the per-layer caches [B, T, 128] (rows < T-1 valid).
     """
+    from .modules import sampling
     te_mod, head = dec.token_emb, dec.lm_head
+    sizes = te_mod.field_sizes
+    bans = _check_filters(top_k, top_p, top_a, banned_tokens, fields, sizes)
     B, T, F = perf.shape
     dev = perf.device
     sw = _StackWeights(dec.transformer)
     table = te_mod.table().detach().contiguous()
     table16 = K.cast_bf16(table)
-    sizes = te_mod.field_sizes
     ln_w, ln_b = te_mod.norm.weight.detach(), te_mod.norm.bias.detach()
     wp16 = K.cast_bf16(te_mod.project_emb.weight.detach().contiguous())
     bp = te_mod.project_emb.bias.detach()
@@ -190,10 +226,22 @@ def render_decoder(dec, perf: Tensor, masked_perf: Tensor, score_hidden: Tensor,
     if K.decode_stack_ok(sw.depth, sw.D, sw.H, sw.layers[0]["w2"].shape[1], sw.ada, style_f.shape[-1], T):
         plan = K.DecodeStackPlan(sw.layers, sw.w_ada, sw.b_ada, kv_caches, B, style_f.shape[-1])
 
-    ks = [top_k if top_k is not None else -(-sizes[f] // 10) for f in fields]
+    filtered = top_p is not None or top_a is not None
+    if filtered:
+        ks = [1] * len(fields)                                                  # ignored by the filtered fields
+    elif not isinstance(top_k, (list, tuple)):
+        ks = [top_k if top_k is not None else -(-sizes[f] // 10) for f in fields]
+    else:
+        ks = [int(k) for k in top_k]
+        assert len(ks) == len(fields), "top_k: one k per rendered field"
     fused_sampling = (generator is None and emb == 128 and len(fields) <= 8 and all(sizes[f] <= 256 for f in fields)
                       and all(1 <= k <= 32 for k in ks) and K._os.environ.get("SPB_DECODE", "fused") == "fused")
-    seed = K.seed_from_torch() if any(k > 1 for k in ks) else 0
+    seed = K.seed_from_torch() if filtered or any(k > 1 for k in ks) else 0
+    # the filters and bans of the sampling launch (all None: the plain top-k call)
+    filt_kw = dict(top_p=None if top_p is None else [float(top_p)] * len(fields),
+                   top_a=None if top_a is None else [(float(top_a[0]), float(top_a[1]))] * len(fields),
+                   banned=bans if any(bans) else None)
+    ban_idx = {f: torch.tensor(ids, dtype=torch.int64, device=dev) for f, ids in zip(fields, bans) if ids}
 
     # Everything of a note-step that does not depend on the tokens sampled so far is evaluated for ALL positions before the loop,
     # in large launches: the masked tuple of note i+1 through the embedding and its half of project_multiemb (+ bias), and the
@@ -255,13 +303,11 @@ def render_decoder(dec, perf: Tensor, masked_perf: Tensor, score_hidden: Tensor,
         e, _, _ = K.layer_norm_fwd(e_raw, hn_w, hn_b, out_dtype=BF16, need_stats=False)
         if front_in_kernel:
             # the sampling kernel's last CTA ends the step: position += 1, grid-barrier word of the stack kernel back to zero
-            K.sample_fields(e, table16, fields, [offs[f] for f in fields], [sizes[f] for f in fields],
-                            [top_k if top_k is not None else -(-sizes[f] // 10) for f in fields], out, pos_t,
-                            temperature=temperature, seed=seed, advance=plan.advance)
+            K.sample_fields(e, table16, fields, [offs[f] for f in fields], [sizes[f] for f in fields], ks, out, pos_t,
+                            temperature=temperature, seed=seed, advance=plan.advance, **filt_kw)
         else:
-            K.sample_fields(e, table16, fields, [offs[f] for f in fields], [sizes[f] for f in fields],
-                            [top_k if top_k is not None else -(-sizes[f] // 10) for f in fields], out, pos_t,
-                            temperature=temperature, seed=seed)
+            K.sample_fields(e, table16, fields, [offs[f] for f in fields], [sizes[f] for f in fields], ks, out, pos_t,
+                            temperature=temperature, seed=seed, **filt_kw)
             pos_t.add_(1)
 
     def step():
@@ -285,17 +331,20 @@ def render_decoder(dec, perf: Tensor, masked_perf: Tensor, score_hidden: Tensor,
         e_raw = K.gemm(K.cast_bf16(hid), whead16, trans_b=True, out_dtype=BF16)
         e, _, _ = K.layer_norm_fwd(e_raw, hn_w, hn_b, out_dtype=BF16, need_stats=False)
         if fused_sampling:
-            # heads of the rendered fields, PAD / MASK ban, top-k filter, draw and token write: one launch
-            K.sample_fields(e, table16, fields, [offs[f] for f in fields], [sizes[f] for f in fields],
-                            [top_k if top_k is not None else -(-sizes[f] // 10) for f in fields], out, pos_t,
-                            temperature=temperature, seed=seed)
+            # heads of the rendered fields, PAD / MASK and per-field bans, logit filter, draw and token write: one launch
+            K.sample_fields(e, table16, fields, [offs[f] for f in fields], [sizes[f] for f in fields], ks, out, pos_t,
+                            temperature=temperature, seed=seed, **filt_kw)
         else:
             toks = []
-            for f in fields:
+            for f, k in zip(fields, ks):
                 lg = K.gemm(e[:, f * emb:(f + 1) * emb], table16[offs[f]:offs[f] + sizes[f]], out_dtype=F32)
                 lg[:, :2] = neg_inf                                             # PAD / MASK are never emitted
-                k = top_k if top_k is not None else -(-sizes[f] // 10)
-                if k == 1:
+                if f in ban_idx:
+                    lg.index_fill_(1, ban_idx[f], neg_inf)
+                if filtered:
+                    lg = sampling.top_p(lg, float(top_p)) if top_p is not None else _top_a_rows(lg, *top_a)
+                    tok = torch.multinomial(torch.softmax(lg / temperature, dim=-1), 1, generator=generator).squeeze(1)
+                elif k == 1:
                     tok = lg.argmax(dim=-1)
                 else:
                     val, ind = torch.topk(lg, k)
@@ -309,7 +358,8 @@ def render_decoder(dec, perf: Tensor, masked_perf: Tensor, score_hidden: Tensor,
         pos_t.add_(1)
 
     n_steps = T - 1 - start
-    graph_ok = use_graph and generator is None and n_steps > 4
+    # host-side filters sort and mask with data-dependent shapes: that step runs eagerly
+    graph_ok = use_graph and generator is None and n_steps > 4 and (fused_sampling or not filtered)
     if not graph_ok:
         for _ in range(n_steps):
             step()
@@ -328,6 +378,15 @@ def render_decoder(dec, perf: Tensor, masked_perf: Tensor, score_hidden: Tensor,
         graph.replay()
     K.LAUNCHES += per_step * (n_steps - 2)       # ... each replay launches every recorded kernel
     return (out, kv_caches) if return_kv else out
+
+
+def _top_a_rows(logits: Tensor, min_p_pow: float, min_p_ratio: float) -> Tensor:
+    """modules.sampling.top_a with the limit taken per row (per score) instead of over the whole [B, V] tensor, as the sampling
+    kernel does; the most probable token is always kept."""
+    probs = torch.softmax(logits, dim=-1)
+    top = probs.max(dim=-1, keepdim=True).values
+    limit = torch.minimum(top.pow(min_p_pow) * min_p_ratio, top)
+    return torch.where(probs < limit, float("-inf"), logits)
 
 
 # ----------------------------------------------------------------------------- reference-signature entry points

@@ -19,6 +19,7 @@ tests/test_inference_host.py replays whole renderings against logs produced by t
 """
 from __future__ import annotations
 
+import math
 from dataclasses import dataclass
 from types import SimpleNamespace
 from typing import Callable, Dict, Optional, Union
@@ -363,21 +364,53 @@ class ScorePerformerGenerator:
         return caches
 
 
+# the reference's logit filters (modules/sampling.py) and the keyword arguments each takes, with its defaults
+_BATCH_FILTERS = {"top_k": {"thres": 0.9, "k": None}, "top_p": {"thres": 0.9}, "top_a": {"min_p_pow": 2.0, "min_p_ratio": 0.02}}
+
+
+def _batch_sampling(filter_logits_fn: Callable, filter_kwargs: Optional[Dict[str, object]], model, cols) -> Dict[str, object]:
+    """`render_batch` keyword arguments for a reference filter function and its kwargs; raises on anything else.  top-k's `thres`
+    gives k = ceil((1 - thres) V) per rendered field, V the vocabulary of the field's head."""
+    from ..modules import sampling
+    name = next((n for n in _BATCH_FILTERS if filter_logits_fn is getattr(sampling, n)), None)
+    if name is None and getattr(filter_logits_fn, "__module__", "").endswith("modules.sampling"):
+        name = getattr(filter_logits_fn, "__name__", None)              # the same functions of the original package
+    if name not in _BATCH_FILTERS:
+        raise ValueError(f"render_performances samples with top_k, top_p or top_a of modules.sampling, not {filter_logits_fn!r}")
+    kw = dict(filter_kwargs or {})
+    unknown = set(kw) - set(_BATCH_FILTERS[name])
+    if unknown:
+        raise ValueError(f"{name} takes {sorted(_BATCH_FILTERS[name])}, not {sorted(unknown)}")
+    args = {**_BATCH_FILTERS[name], **kw}
+    if name == "top_p":
+        return {"top_p": float(args["thres"])}
+    if name == "top_a":
+        return {"top_a": (float(args["min_p_pow"]), float(args["min_p_ratio"]))}
+    if args["k"] is not None or "thres" not in kw:
+        return {"top_k": args["k"]}                                      # None: render_batch's ceil(0.1 V), the reference default
+    sizes = model.perf_decoder.model.token_emb.field_sizes
+    return {"top_k": [math.ceil((1 - float(args["thres"])) * sizes[c]) for c in cols]}
+
+
 def render_performances(model, messenger: SPMupleMessenger, collator, pieces, filter_kwargs: Optional[Dict[str, object]] = None,
-                        temperature: float = 1., time_messages: bool = True, sort_messages: bool = True):
+                        temperature: float = 1., time_messages: bool = True, sort_messages: bool = True,
+                        filter_logits_fn: Callable = top_k):
     """Whole pieces, many at once: the offline counterpart of the window loop (SURVEY §8 C5 -- the reference renders one piece at a
     time through the same loop with an infinite window).  `pieces` are `PerformanceData` as `prepare_performance_notes` leaves them
     (notes with the rendered fields MASKed, per-note score / style embeddings, messenger state); pieces must fit the decoder context
     as a whole (no truncation happens here).  All pieces advance in lock-step through `decode.render_batch` -- one persistent
     decoder-stack launch and one heads + sampling launch per note for the whole batch -- then the rendered tuples come back in ONE
-    device->host copy and each piece goes through the messenger.  Sampling is top-k (`filter_kwargs={'k': k}`, default ceil(0.1 V) as
-    in modules/sampling.py:28-59).  Returns `[(gen_seq, messages), ...]` and completes every piece's `gen_seq` / `intermediates`."""
+    device->host copy and each piece goes through the messenger.  Sampling takes the reference's filters: `filter_logits_fn` is `top_k`
+    (`filter_kwargs` `k` or `thres`; default ceil(0.1 V)), `top_p` (`thres`) or `top_a` (`min_p_pow`, `min_p_ratio`) of
+    modules/sampling.py with their defaults; any other function or keyword raises ValueError.  top-a takes each piece's own
+    largest probability (the reference's takes it over the batch it is given, here one piece).  Returns `[(gen_seq, messages), ...]` and completes every piece's `gen_seq` / `intermediates`."""
     from ..decode import render_batch
     tok = messenger.tokenizer
     if not pieces or any(pd.notes is None or pd.context is None or pd.embeddings is None for pd in pieces):
         raise ValueError("render_performances needs notes, score embeddings (context) and style embeddings for every piece")
     sos, eos = tok[0, SOS_TOKEN], tok[0, EOS_TOKEN]
     cols = sorted(set(range(len(tok.sizes))).difference(collator.mask_ignore_token_dims))
+    sampling_kw = _batch_sampling(filter_logits_fn, filter_kwargs, model, cols)
     dev = pieces[0].context.device
     rows = []
     for pd in pieces:
@@ -399,9 +432,8 @@ def render_performances(model, messenger: SPMupleMessenger, collator, pieces, fi
     masked = tokens.copy()
     for i, (notes, first) in enumerate(rows):
         masked[i, first:notes.shape[0]][:, cols] = collator.mask_token_id
-    k = None if not filter_kwargs else filter_kwargs.get("k")
     out = render_batch(model, torch.from_numpy(tokens).to(dev), torch.from_numpy(masked).to(dev), context, style,
-                       mask=torch.from_numpy(valid).to(dev), fields=cols, temperature=temperature, top_k=k)
+                       mask=torch.from_numpy(valid).to(dev), fields=cols, temperature=temperature, **sampling_kw)
     host = out.cpu().numpy()
     results = []
     for i, ((notes, first), pd) in enumerate(zip(rows, pieces)):

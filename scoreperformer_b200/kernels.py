@@ -5,7 +5,7 @@ entry point launches, so bench.py can report `gpu_launches`.
 """
 from __future__ import annotations
 
-from typing import Optional, Sequence
+from typing import Optional, Sequence, Tuple
 
 import ctypes
 import torch
@@ -243,10 +243,15 @@ def gather_at_pos(srcs: Sequence[Tensor], dsts: Sequence[Tensor], shifts: Sequen
 
 def sample_fields(e: Tensor, table16: Tensor, fields: Sequence[int], offsets: Sequence[int], vocab: Sequence[int], topk: Sequence[int],
                   tokens: Tensor, pos_dev: Tensor, temperature: float = 1.0, seed: int = 0, n_banned: int = 2,
-                  advance: Optional[Tensor] = None) -> None:
+                  advance: Optional[Tensor] = None, top_p: Optional[Sequence[float]] = None,
+                  top_a: Optional[Sequence[Optional[Tuple[float, float]]]] = None,
+                  banned: Optional[Sequence[Sequence[int]]] = None) -> None:
     """Heads of `fields` + top-k sampling (k = 1: greedy) + write of tokens[:, pos + 1, field], one launch (csrc/decode_stack.cu).
     `advance` (int32 [2], [0] zero): the last CTA also does pos += 1 and clears both words (DecodeStackPlan.barrier is laid out so that
-    advance[1] is the stack kernel's grid-barrier word)."""
+    advance[1] is the stack kernel's grid-barrier word).
+    Per field (one entry per listed field; None = off for all): `top_p` thresholds (None or < 0: off), `top_a` (min_p_pow,
+    min_p_ratio) pairs (None: off) and `banned` token ids never emitted besides [0, n_banned).  A field with a top-p / top-a filter
+    ignores its k.  Without any of the three this is exactly the spb_sample_fields call."""
     import ctypes
     _require_cuda(e, table16, tokens)
     assert e.dtype == BF16 and e.stride(1) == 1 and table16.dtype == BF16 and table16.is_contiguous() and table16.shape[1] == 128
@@ -254,8 +259,26 @@ def sample_fields(e: Tensor, table16: Tensor, fields: Sequence[int], offsets: Se
     n = len(fields)
     arr = lambda xs: (ctypes.c_int * n)(*[int(x) for x in xs])
     B, T, F = tokens.shape
-    _call("spb_sample_fields", _p(e), e.stride(0), _p(table16), arr(fields), arr(offsets), arr(vocab), arr(topk), n, int(n_banned),
-          float(temperature), int(seed), _p(pos_dev), _p(tokens), B, T, F, _p(advance), _stream())
+    args = (_p(e), e.stride(0), _p(table16), arr(fields), arr(offsets), arr(vocab), arr(topk), n, int(n_banned), float(temperature),
+            int(seed), _p(pos_dev), _p(tokens), B, T, F, _p(advance))
+    if top_p is None and top_a is None and banned is None:
+        _call("spb_sample_fields", *args, _stream())
+    else:
+        farr = lambda xs: None if xs is None else (ctypes.c_float * n)(*[float(x) for x in xs])
+        assert all(len(x) == n for x in (top_p, top_a, banned) if x is not None)
+        pp = None if top_p is None else [-1.0 if t is None else t for t in top_p]
+        a_pow = None if top_a is None else [0.0 if a is None else a[0] for a in top_a]
+        a_ratio = None if top_a is None else [0.0 if a is None else a[1] for a in top_a]
+        bits = None
+        if banned is not None:
+            words = [0] * (8 * n)
+            for i, ids in enumerate(banned):
+                for v in ids:
+                    v = int(v)
+                    assert 0 <= v < 256, f"banned token {v} is outside 0..255"
+                    words[8 * i + v // 32] |= 1 << (v % 32)
+            bits = (ctypes.c_uint32 * (8 * n))(*words)
+        _call("spb_sample_fields_filtered", *args, farr(pp), farr(a_pow), farr(a_ratio), bits, _stream())
     _count()
 
 

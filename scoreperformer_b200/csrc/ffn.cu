@@ -3,21 +3,25 @@
 // Reference: modules/transformer/feedforward.py:13-22 (GLU), :35-64 (FeedForward: proj -> GLU -> dropout -> out) and the
 // pre-norm residual around it, modules/transformer/transformer.py:139-232.
 //
-// One persistent CTA per SM owns 128 rows (note-tuples) at a time and streams the two weight matrices through shared memory in
-// chunks of 64 hidden units; the [128 x 2048] pre-activation and the [128 x 1024] hidden activation never exist as a whole:
-//   GEMM1(c)  u_c[128 x 128]   = xn[128 x 256] . W1_c^T      W1_c = value rows [64c, 64c+64) and gate rows [1024+64c, ..) stacked;
+// A CTA pair (cluster of two, tcgen05 cta_group::2) owns 256 rows (note-tuples) at a time, 128 per CTA, and walks the tiles
+// persistently.  The two weight matrices stream through shared memory in chunks of 64 hidden units; the [256 x 2048]
+// pre-activation and the [256 x 1024] hidden activation never exist as a whole:
+//   GEMM1(c)  u_c[256 x 128]   = xn[256 x 256] . W1_c^T      W1_c = value rows [64c, 64c+64) and gate rows [1024+64c, ..) stacked;
 //                                                             xn stays resident in smem for the 16 chunks; accumulator in TMEM
-//   GLU(c)    h_c[128 x 64]    = (u_val + b) * silu(u_gate + b) * keep      8 epilogue warps, one row per thread (TMEM lane == row),
-//                                                             bf16 into a 128B-swizzled smem tile = the A operand of GEMM2
-//   GEMM2(c)  acc[128 x 256]  += h_c[128 x 64] . W2[:, 64c:64c+64]^T         accumulates in TMEM over the 16 chunks
+//   GLU(c)    h_c[256 x 64]    = (u_val + b) * silu(u_gate + b) * keep      16 epilogue warps per CTA, one row per thread
+//                                                             (TMEM lane == row), bf16 into a 128B-swizzled smem tile = the A
+//                                                             operand of GEMM2
+//   GEMM2(c)  acc[256 x 256]  += h_c[256 x 64] . W2[:, 64c:64c+64]^T         accumulates in TMEM over the 16 chunks
 //   out       = acc + resid                                                   fp32, once per tile
-// The MMA thread issues GEMM1(c+1) before GEMM2(c), so the tensor pipe works on the next chunk while the epilogue warps run the
-// GLU of this one (u is double-buffered in TMEM: 256 + 2 x 128 = 512 columns).
-// For the backward (ffn_bwd.cu consumes u, the dW2 weight-gradient GEMM consumes h) the kernel can also emit u (bf16 [n, 2048], bias
-// included) and h (bf16 [n, 1024]).
-// HBM traffic per row: 512 B (xn) + 1 KB (resid) + 1 KB (out) [+ 4 KB u + 2 KB h when saved]; the weights (1.5 MB) stream from L2.
+// Each CTA stages its own 128 rows of xn / h and only HALF of every weight tile (CTA 0 the value rows of W1_c and output rows
+// [0,128) of W2, CTA 1 the gate rows and output rows [128,256)), so the 1.5 MB of weights stream out of L2 once per 256 rows, and
+// one tcgen05.mma issued by the leader CTA drives both SMs' tensor cores.  The leader issues GEMM1(c+1) before GEMM2(c), so the
+// tensor pipe works on the next chunk while the epilogue warps run the GLU of this one (u is double-buffered in TMEM:
+// 256 + 2 x 128 = 512 columns).
+// For the backward (ffn_bwd.cu consumes u, the dW2 weight-gradient GEMM consumes h) the kernel can also emit u (bf16 [n, 2048],
+// bias included) and h (bf16 [n, 1024]); both leave through TMA stores from staging tiles as whole 128-byte lines.
+// HBM traffic per row: 512 B (xn) + 1 KB (resid) + 1 KB (out) [+ 4 KB u + 2 KB h when saved].
 #include "attention_tc.cuh"
-#include <stdlib.h>
 #include <string.h>
 
 namespace {
@@ -25,23 +29,12 @@ using attn_tc::tmem_ld_32x32b_x16;
 
 constexpr int D = 256;            // model width
 constexpr int HID = 1024;         // hidden units (GLU: W1 has 2 * HID rows)
-constexpr int BMF = 128;          // rows per tile
+constexpr int BMF = 128;          // rows per CTA (a tile of the pair is 2 x BMF rows)
 constexpr int CH = 64;            // hidden units per chunk
 constexpr int NCH = HID / CH;     // 16 chunks
 constexpr int KB1 = D / 64;       // 4 k-blocks of GEMM1
-constexpr int W1_STAGES = 4;      // ring of [128 rows (64 value + 64 gate) x 64 k] tiles, 16 KB each
-constexpr int W2_STAGES = 2;      // ring of [256 rows x 64 k] tiles, 32 KB each
-constexpr int SA_OFF = 0;                                  // xn tile: KB1 x [128 x 64]                 64 KB
-constexpr int SW1_OFF = SA_OFF + KB1 * 16384;              //                                           64 KB
-constexpr int SW2_OFF = SW1_OFF + W1_STAGES * 16384;       //                                           64 KB
-constexpr int SH_OFF = SW2_OFF + W2_STAGES * 32768;        // h chunks: 2 x [128 x 64]                  32 KB
-constexpr int SBIAS_OFF = SH_OFF + 2 * 16384;              // per lane quarter: 2 x 64 floats            2 KB
-constexpr int BAR_OFF = SBIAS_OFF + 4 * 512;
-constexpr int FFN_SMEM_BYTES = BAR_OFF + 256;
-static_assert(FFN_SMEM_BYTES <= 232448, "exceeds the 227 KB of shared memory a CTA may have");
-constexpr int EPQ = 4;                    // epilogue warps per TMEM lane quarter
+constexpr int EPQ = 4;            // epilogue warps per TMEM lane quarter
 constexpr int FFN_EPI_WARPS = 4 * EPQ;
-constexpr int FFN_THREADS = 96 + FFN_EPI_WARPS * 32;        // TMA producer, GEMM1 issuer, GEMM2 issuer, epilogue warps
 constexpr uint32_t TM_OUT = 0, TM_U = 256;
 
 struct FfnParams {
@@ -59,301 +52,6 @@ struct FfnParams {
     float keep_scale;
 };
 
-__global__ void __launch_bounds__(FFN_THREADS, 1)
-ffn_fwd_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CUtensorMap tmW1, const __grid_constant__ CUtensorMap tmW2,
-               FfnParams p) {
-    extern __shared__ __align__(1024) uint8_t smem[];
-    uint64_t* bars = reinterpret_cast<uint64_t*>(smem + BAR_OFF);
-    uint64_t* a_full = bars + 0;
-    uint64_t* a_empty = bars + 1;
-    uint64_t* w1_full = bars + 2;          // [W1_STAGES]
-    uint64_t* w1_empty = bars + 6;
-    uint64_t* w2_full = bars + 10;         // [W2_STAGES]
-    uint64_t* w2_empty = bars + 12;
-    uint64_t* u_full = bars + 14;          // [2]  u chunk is in TMEM buffer b
-    uint64_t* u_empty = bars + 16;         // [2]  ... and has been read out (8 warps)
-    uint64_t* h_full = bars + 18;          // [2]  h chunk is in smem buffer b (8 warps)
-    uint64_t* h_empty = bars + 20;         // [2]  ... and GEMM2 has consumed it
-    uint64_t* out_full = bars + 22;
-    uint64_t* out_empty = bars + 23;       // output accumulator read out (8 warps)
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 24);
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int n_tiles = (p.n_rows + BMF - 1) / BMF;
-
-    if (threadIdx.x == 0) {
-        if ((smem_u32(smem) & 1023u) != 0) {
-            printf("spb200: ffn_fwd_kernel needs 1024-byte aligned dynamic shared memory\n");
-            __trap();
-        }
-        tma_prefetch_desc(&tmX);
-        tma_prefetch_desc(&tmW1);
-        tma_prefetch_desc(&tmW2);
-        mbar_init(a_full, 1); mbar_init(a_empty, 1);
-        for (int s = 0; s < W1_STAGES; ++s) { mbar_init(&w1_full[s], 1); mbar_init(&w1_empty[s], 1); }
-        for (int s = 0; s < W2_STAGES; ++s) { mbar_init(&w2_full[s], 1); mbar_init(&w2_empty[s], 1); }
-        for (int b = 0; b < 2; ++b) {
-            mbar_init(&u_full[b], 1); mbar_init(&u_empty[b], FFN_EPI_WARPS);
-            mbar_init(&h_full[b], FFN_EPI_WARPS); mbar_init(&h_empty[b], 1);
-        }
-        mbar_init(out_full, 1); mbar_init(out_empty, FFN_EPI_WARPS);
-        fence_mbar_init();
-    }
-    if (warp == 1) tmem_alloc<512>(tmem_slot);
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot;
-
-    if (warp == 0) {
-        // ------------------------------------------------------------------ TMA producer
-        if (lane == 0) {
-            int s1 = 0;
-            uint32_t ph1 = 0;
-            int it = 0;
-            for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, ++it) {
-                const int m0 = tile * BMF;
-                auto load_w1 = [&](int c) {
-                    for (int kb = 0; kb < KB1; ++kb) {
-                        SPB_MBAR_WAIT(&w1_empty[s1], ph1 ^ 1u);
-                        mbar_arrive_expect_tx(&w1_full[s1], 16384);
-                        uint8_t* dst = smem + SW1_OFF + s1 * 16384;
-                        tma_load_2d(dst, &tmW1, &w1_full[s1], kb * 64, c * CH);                // value rows
-                        tma_load_2d(dst + 8192, &tmW1, &w1_full[s1], kb * 64, HID + c * CH);   // gate rows
-                        if (++s1 == W1_STAGES) { s1 = 0; ph1 ^= 1u; }
-                    }
-                };
-                load_w1(0);                                    // does not depend on the previous tile's xn being released
-                SPB_MBAR_WAIT(a_empty, (uint32_t)(it & 1) ^ 1u);
-                mbar_arrive_expect_tx(a_full, KB1 * 16384);
-#pragma unroll
-                for (int kb = 0; kb < KB1; ++kb) tma_load_2d(smem + SA_OFF + kb * 16384, &tmX, a_full, kb * 64, m0);
-                for (int c = 0; c < NCH; ++c) {
-                    if (c > 0) load_w1(c);
-                    const int g = it * NCH + c, s2 = g & 1;
-                    SPB_MBAR_WAIT(&w2_empty[s2], (uint32_t)((g >> 1) & 1) ^ 1u);
-                    mbar_arrive_expect_tx(&w2_full[s2], 32768);
-                    tma_load_2d(smem + SW2_OFF + s2 * 32768, &tmW2, &w2_full[s2], c * CH, 0);
-                }
-            }
-        }
-    } else if (warp == 1) {
-        // ------------------------------------------------------------------ GEMM1 issuer: u chunks, one ahead of the epilogue
-        // (a tcgen05.mma costs its issuing thread ~60 cycles whatever its shape, so the two GEMMs get a thread each)
-        if (lane == 0) {
-            constexpr uint32_t idesc1 = umma_idesc_bf16(BMF, 2 * CH, false, false);
-            const uint32_t sa = smem_u32(smem + SA_OFF), sw1 = smem_u32(smem + SW1_OFF);
-            int s1 = 0;
-            uint32_t ph1 = 0;
-            int it = 0;
-            for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, ++it) {
-                SPB_MBAR_WAIT(a_full, (uint32_t)(it & 1));
-                for (int c = 0; c < NCH; ++c) {
-                    const int g = it * NCH + c, b = g & 1;
-                    SPB_MBAR_WAIT(&u_empty[b], (uint32_t)((g >> 1) & 1) ^ 1u);
-                    tc_fence_after();
-                    for (int kb = 0; kb < KB1; ++kb) {
-                        SPB_MBAR_WAIT(&w1_full[s1], ph1);
-                        tc_fence_after();
-#pragma unroll
-                        for (int k = 0; k < 4; ++k)
-                            umma_bf16(tmem_base + TM_U + b * 128, umma_smem_desc_sw128(sa + kb * 16384 + k * 32, 0, 1024),
-                                      umma_smem_desc_sw128(sw1 + s1 * 16384 + k * 32, 0, 1024), idesc1, (kb > 0 || k > 0) ? 1u : 0u);
-                        umma_commit(&w1_empty[s1]);
-                        if (++s1 == W1_STAGES) { s1 = 0; ph1 ^= 1u; }
-                    }
-                    umma_commit(&u_full[b]);
-                }
-                umma_commit(a_empty);                      // every GEMM1 of this tile has been issued: xn may be replaced
-            }
-        }
-    } else if (warp == 2) {
-        // ------------------------------------------------------------------ GEMM2 issuer: acc += h_c W2_c^T as each h chunk arrives
-        if (lane == 0) {
-            constexpr uint32_t idesc2 = umma_idesc_bf16(BMF, D, false, false);
-            const uint32_t sw2 = smem_u32(smem + SW2_OFF), sh = smem_u32(smem + SH_OFF);
-            int it = 0;
-            for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, ++it) {
-                for (int c = 0; c < NCH; ++c) {
-                    const int g = it * NCH + c, b = g & 1;
-                    SPB_MBAR_WAIT(&h_full[b], (uint32_t)((g >> 1) & 1));
-                    SPB_MBAR_WAIT(&w2_full[b], (uint32_t)((g >> 1) & 1));
-                    if (c == 0) SPB_MBAR_WAIT(out_empty, (uint32_t)(it & 1) ^ 1u);
-                    tc_fence_after();
-#pragma unroll
-                    for (int k = 0; k < 4; ++k)
-                        umma_bf16(tmem_base + TM_OUT, umma_smem_desc_sw128(sh + b * 16384 + k * 32, 0, 1024),
-                                  umma_smem_desc_sw128(sw2 + b * 32768 + k * 32, 0, 1024), idesc2, (c > 0 || k > 0) ? 1u : 0u);
-                    umma_commit(&w2_empty[b]);
-                    umma_commit(&h_empty[b]);
-                }
-                umma_commit(out_full);
-            }
-        }
-    } else {
-        // ------------------------------------------------------------------ epilogue warps: thread == row (TMEM lane); the EPQ warps
-        // of a lane quarter split the chunk's 64 hidden units (and the output's 256 columns) evenly
-        constexpr int HW = CH / EPQ;                       // hidden units per warp and chunk
-        constexpr int UW = EPQ == 2 ? 32 : 16;             // output columns per unit (4 units per warp)
-        const int ew = warp - 3;
-        const int q = warp & 3;                            // TMEM lane quarter this warp may touch
-        const int part = ew >> 2;                          // which slice of the quarter's columns
-        const uint32_t lane_addr = (uint32_t)(q * 32) << 16;
-        const int r = q * 32 + lane;                       // row inside the tile
-        float* sbias = reinterpret_cast<float*>(smem + SBIAS_OFF + ew * (2 * HW * 4));      // [value HW | gate HW], 16-byte aligned
-        uint64_t seed = p.seed;
-        if (p.rng_offset != nullptr) seed += *p.rng_offset * 0x9E3779B97F4A7C15ull;
-        const uint32_t seed32 = spb_seed32(seed);
-        const bool drop_on = p.thr32 != 0;
-        const uint32_t sh_row = smem_u32(smem + SH_OFF) + (uint32_t)(r * 128);
-        const uint32_t swz = (uint32_t)(r & 7);
-        int it = 0;
-        // bias element (chunk c, slot i): i < HW value, else gate; each lane fetches slots lane, lane + 32 one chunk ahead
-        auto bias_at = [&](int c, int i) -> float {
-            return i < 2 * HW ? __ldg(p.bias1 + (i < HW ? 0 : HID - HW) + c * CH + part * HW + i) : 0.f;
-        };
-        float bias_a = bias_at(0, lane), bias_b = bias_at(0, lane + 32);
-        for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, ++it) {
-            const int row = tile * BMF + r;
-            const bool row_ok = row < p.n_rows;
-            for (int c = 0; c < NCH; ++c) {
-                const int g = it * NCH + c, b = g & 1;
-                const uint32_t ph = (uint32_t)((g >> 1) & 1);
-                const int hid0 = c * CH + part * HW;       // first hidden unit of this warp's slice
-                __syncwarp();
-                if (lane < 2 * HW) sbias[lane] = bias_a;
-                if (lane + 32 < 2 * HW) sbias[lane + 32] = bias_b;
-                __syncwarp();
-                {
-                    const int cn = (c + 1 < NCH) ? c + 1 : 0;
-                    bias_a = bias_at(cn, lane);
-                    bias_b = bias_at(cn, lane + 32);
-                }
-                SPB_MBAR_WAIT(&u_full[b], ph);
-                tc_fence_after();
-                uint32_t val[HW], gat[HW];
-                if (HW == 32) {
-                    tmem_ld_32x32b_x32(tmem_base + TM_U + b * 128 + lane_addr + part * HW, val);
-                    tmem_ld_32x32b_x32(tmem_base + TM_U + b * 128 + lane_addr + 64 + part * HW, gat);
-                } else {
-                    tmem_ld_32x32b_x16(tmem_base + TM_U + b * 128 + lane_addr + part * HW, val);
-                    tmem_ld_32x32b_x16(tmem_base + TM_U + b * 128 + lane_addr + 64 + part * HW, gat);
-                }
-                tmem_ld_wait();
-                tc_fence_before();
-                __syncwarp();
-                if (lane == 0) mbar_arrive(&u_empty[b]);
-                uint32_t hp[HW / 2];
-                const uint32_t quad0 = (uint32_t)row * (uint32_t)(HID >> 2) + (uint32_t)(hid0 >> 2);
-                const float4* sb4 = reinterpret_cast<const float4*>(sbias);
-#pragma unroll
-                for (int j = 0; j < HW; j += 4) {
-                    const float4 bv = sb4[j >> 2], bg = sb4[(HW >> 2) + (j >> 2)];       // one broadcast read per four columns
-                    const float bvs[4] = {bv.x, bv.y, bv.z, bv.w}, bgs[4] = {bg.x, bg.y, bg.z, bg.w};
-                    float o[4];
-#pragma unroll
-                    for (int e = 0; e < 4; ++e) {
-                        const float v = __uint_as_float(val[j + e]) + bvs[e];
-                        const float gt = __uint_as_float(gat[j + e]) + bgs[e];
-                        val[j + e] = __float_as_uint(v);
-                        gat[j + e] = __float_as_uint(gt);
-                        // silu(g) = g * sigmoid(g) = g/2 * (1 + tanh(g/2)): one MUFU instead of exp + reciprocal
-                        const float hg = 0.5f * gt;
-                        float th;
-                        asm("tanh.approx.f32 %0, %1;" : "=f"(th) : "f"(hg));
-                        o[e] = v * fmaf(hg, th, hg);
-                    }
-                    if (drop_on) {         // same mask function as glu_fwd_kernel / glu_bwd_kernel (rowops.cu)
-                        const uint32_t qh = spb_quad_hash(seed32, quad0 + (uint32_t)(j >> 2));
-#pragma unroll
-                        for (int e = 0; e < 4; ++e) o[e] = spb_quad_keep(qh, e, p.thr32) ? o[e] * p.keep_scale : 0.f;
-                    }
-                    hp[j >> 1] = pack_bf16x2(o[0], o[1]);
-                    hp[(j >> 1) + 1] = pack_bf16x2(o[2], o[3]);
-                }
-                if (p.u_save != nullptr && row_ok) {
-                    __nv_bfloat16* uv = p.u_save + (size_t)row * (2 * HID) + hid0;
-#pragma unroll
-                    for (int j = 0; j < HW; j += 8) {
-                        *reinterpret_cast<uint4*>(uv + j) =
-                            make_uint4(pack_bf16x2(__uint_as_float(val[j]), __uint_as_float(val[j + 1])),
-                                       pack_bf16x2(__uint_as_float(val[j + 2]), __uint_as_float(val[j + 3])),
-                                       pack_bf16x2(__uint_as_float(val[j + 4]), __uint_as_float(val[j + 5])),
-                                       pack_bf16x2(__uint_as_float(val[j + 6]), __uint_as_float(val[j + 7])));
-                        *reinterpret_cast<uint4*>(uv + HID + j) =
-                            make_uint4(pack_bf16x2(__uint_as_float(gat[j]), __uint_as_float(gat[j + 1])),
-                                       pack_bf16x2(__uint_as_float(gat[j + 2]), __uint_as_float(gat[j + 3])),
-                                       pack_bf16x2(__uint_as_float(gat[j + 4]), __uint_as_float(gat[j + 5])),
-                                       pack_bf16x2(__uint_as_float(gat[j + 6]), __uint_as_float(gat[j + 7])));
-                    }
-                }
-                if (p.h_save != nullptr && row_ok) {
-                    __nv_bfloat16* hv = p.h_save + (size_t)row * HID + hid0;
-#pragma unroll
-                    for (int j = 0; j < HW / 8; ++j)
-                        *reinterpret_cast<uint4*>(hv + j * 8) = make_uint4(hp[4 * j], hp[4 * j + 1], hp[4 * j + 2], hp[4 * j + 3]);
-                }
-                SPB_MBAR_WAIT(&h_empty[b], ph ^ 1u);           // GEMM2 of the chunk that last used this buffer has completed
-#pragma unroll
-                for (int j = 0; j < HW / 8; ++j)
-                    sts_u4(sh_row + (uint32_t)(b * 16384) + ((((uint32_t)(part * (HW / 8) + j)) ^ swz) << 4),
-                           make_uint4(hp[4 * j], hp[4 * j + 1], hp[4 * j + 2], hp[4 * j + 3]));
-                fence_proxy_async();
-                __syncwarp();
-                if (lane == 0) mbar_arrive(&h_full[b]);
-            }
-            // ---- output: acc + resid -> fp32, this warp's 256 / EPQ columns of its 32 rows.  A thread owns a whole row, so its
-            // residual reads are whole lines of its own: they are issued one unit ahead (the first before the accumulator is even
-            // complete) and wait in registers.
-            const bool use_res = p.resid != nullptr && row_ok;
-            const float* rs = p.resid + (size_t)(row_ok ? row : 0) * p.ld_res + part * (D / EPQ);
-            float* dst = p.out + (size_t)(row_ok ? row : 0) * p.ld_out + part * (D / EPQ);
-            float4 rbuf[2][UW / 4];
-            auto fetch_res = [&](int cu, float4 (&rb)[UW / 4]) {
-#pragma unroll
-                for (int j = 0; j < UW / 4; ++j)
-                    rb[j] = use_res ? __ldg(reinterpret_cast<const float4*>(rs + cu * UW) + j) : make_float4(0.f, 0.f, 0.f, 0.f);
-            };
-            fetch_res(0, rbuf[0]);
-            SPB_MBAR_WAIT(out_full, (uint32_t)(it & 1));
-            tc_fence_after();
-#pragma unroll
-            for (int cu = 0; cu < 4; ++cu) {
-                if (cu + 1 < 4) fetch_res(cu + 1, rbuf[(cu + 1) & 1]);
-                uint32_t v[UW];
-                if (UW == 32) tmem_ld_32x32b_x32(tmem_base + TM_OUT + lane_addr + part * (D / EPQ) + cu * UW, v);
-                else tmem_ld_32x32b_x16(tmem_base + TM_OUT + lane_addr + part * (D / EPQ) + cu * UW, v);
-                tmem_ld_wait();
-                if (cu == 3) {
-                    tc_fence_before();
-                    __syncwarp();
-                    if (lane == 0) mbar_arrive(out_empty);
-                }
-                if (row_ok) {
-#pragma unroll
-                    for (int j = 0; j < UW / 4; ++j) {
-                        const float4 rr = rbuf[cu & 1][j];
-                        *reinterpret_cast<float4*>(dst + cu * UW + j * 4) =
-                            make_float4(__uint_as_float(v[4 * j]) + rr.x, __uint_as_float(v[4 * j + 1]) + rr.y,
-                                        __uint_as_float(v[4 * j + 2]) + rr.z, __uint_as_float(v[4 * j + 3]) + rr.w);
-                    }
-                }
-            }
-        }
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 1) tmem_dealloc<512>(tmem_base);
-}
-
-
-// ============================================================================================================================
-// CTA-pair version (cta_group::2): the two CTAs of a cluster own 256 rows together.  Each stages ITS 128 rows of xn / h and only
-// HALF of every weight tile (CTA 0 the value rows of W1_c and output rows [0,128) of W2, CTA 1 the gate rows and output rows
-// [128,256)), so the weights stream out of L2 once per 256 rows -- the single-CTA kernel above is bound by exactly that stream
-// (1.5 MB per 128 rows, ~7 TB/s over the chip) -- and one issued tcgen05.mma drives both SMs' tensor cores.  The smem saved on
-// weight stages buys a deeper W1 ring and a staging tile from which u (and h, straight from its operand tile) leave through TMA
-// stores as whole 128-byte lines.
 constexpr int PW1_STAGES = 4;     // [64 rows x 64 k] 8 KB
 constexpr int PW2_STAGES = 2;     // [128 rows x 64 k] 16 KB
 constexpr int P_SA_OFF = 0;                                   // xn tile (own 128 rows)      64 KB
@@ -721,18 +419,6 @@ extern "C" int spb_ffn_fwd(const void* xn, int ld_xn, const void* w1, const floa
     if (rc != SPB_OK) return rc;
     rc = spb_make_tmap_bf16_2d(&tmW1, w1, (uint64_t)D, (uint64_t)(2 * HID), (uint64_t)D * 2, 64, CH);
     if (rc != SPB_OK) return rc;
-    const char* mode = getenv("SPB_FFN_KERNEL");
-    const bool single = mode != nullptr && mode[0] == 's';      // "single": the one-CTA-per-tile kernel, kept for comparison
-    if (single) {
-        rc = spb_make_tmap_bf16_2d(&tmW2, w2, (uint64_t)HID, (uint64_t)D, (uint64_t)HID * 2, 64, D);
-        if (rc != SPB_OK) return rc;
-        SPB_CHECK_CUDA(cudaFuncSetAttribute(ffn_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, FFN_SMEM_BYTES));
-        const int n_tiles = ceil_div(n_rows, BMF);
-        const int grid = n_tiles < spb_num_sms() ? n_tiles : spb_num_sms();
-        ffn_fwd_kernel<<<grid, FFN_THREADS, FFN_SMEM_BYTES, stream>>>(tmX, tmW1, tmW2, p);
-        SPB_CHECK_LAUNCH();
-        return SPB_OK;
-    }
     SPB_CHECK_ARG((u_save == nullptr) == (h_save == nullptr), "spb_ffn_fwd: u_save and h_save come together");
     rc = spb_make_tmap_bf16_2d(&tmW2, w2, (uint64_t)HID, (uint64_t)D, (uint64_t)HID * 2, 64, BMF);
     if (rc != SPB_OK) return rc;

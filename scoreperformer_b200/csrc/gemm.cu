@@ -49,16 +49,13 @@ struct GemmParams {
     int tma_epi;             // 1: C (and the residual) go through TMA boxes; 0: direct vector stores
 };
 
-// NCTA = 2: a CTA pair (cluster of two SMs of one TPC) computes a 256 x BN tile with tcgen05.mma.cta_group::2 -- each CTA
-// stages its own 128 rows of A and only HALF of the B tile, which halves the L2->SM operand traffic per output and leaves
-// room for deeper rings.
-template <int BN, int NCTA>
+template <int BN>
 __host__ __device__ constexpr int gemm_stages() {
-    return NCTA == 2 ? (BN == 256 ? 4 : 6) : (BN == 256 ? 3 : (BN == 128 ? 4 : 6));
+    return BN == 256 ? 3 : (BN == 128 ? 4 : 6);
 }
-template <int BN, int NCTA>
+template <int BN>
 constexpr int gemm_smem_bytes() {
-    return gemm_stages<BN, NCTA>() * (A_STAGE_BYTES + BN / NCTA * BK * 2) + EPI_BYTES + 1024 /*align slack*/ + 512 /*barriers*/;
+    return gemm_stages<BN>() * (A_STAGE_BYTES + BN * BK * 2) + EPI_BYTES + 1024 /*align slack*/ + 512 /*barriers*/;
 }
 
 // Tile walk of one role: t = t0, t0 + step, ... decoded as (split, m-tile, n-tile) with n fastest.  The coordinates advance by
@@ -89,15 +86,13 @@ struct TileWalk {
 // Persistent, warp-specialised GEMM: one CTA per SM walks the tile list (n fastest, so co-running CTAs share the A panel in
 // L2).  The TMA producer and the MMA issuer run ahead across tile boundaries; the accumulator is double-buffered in TMEM
 // (2 x BN columns), so the epilogue of tile i overlaps the main loop of tile i+1.
-template <int BN, bool A_MN, bool B_MN, int NCTA>
+template <int BN, bool A_MN, bool B_MN>
 __global__ void __launch_bounds__(GEMM_THREADS, 1)
 gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                  const __grid_constant__ CUtensorMap tmC, const __grid_constant__ CUtensorMap tmR, GemmParams p) {
-    constexpr int BN_CTA = BN / NCTA;            // rows of B staged by one CTA
-    constexpr int BM_TILE = BM * NCTA;           // rows of C per (pair) tile
-    constexpr int B_STAGE_BYTES = BN_CTA * BK * 2;
+    constexpr int B_STAGE_BYTES = BN * BK * 2;
     constexpr int STAGE_BYTES = A_STAGE_BYTES + B_STAGE_BYTES;
-    constexpr int STAGES = gemm_stages<BN, NCTA>();
+    constexpr int STAGES = gemm_stages<BN>();
     constexpr int TMEM_COLS = 2 * BN;            // double-buffered accumulator (BN = 256 uses all 512 columns)
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -112,12 +107,11 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
     const int warp = threadIdx.x >> 5;
     const int lane = threadIdx.x & 31;
     const int tiles_n = (p.N + BN - 1) / BN;
-    const int tiles_m = (p.M + BM_TILE - 1) / BM_TILE;
+    const int tiles_m = (p.M + BM - 1) / BM;
     const int tiles_mn = tiles_m * tiles_n;
     const int total_tiles = tiles_mn * p.splits;
     const int total_kb = (p.K + BK - 1) / BK;
-    const int rank = NCTA == 2 ? (int)cluster_ctarank() : 0;         // 0 = leader: issues the MMAs, owns the gating barriers
-    const int tile0 = blockIdx.x / NCTA, tile_step = gridDim.x / NCTA;
+    const int tile0 = blockIdx.x, tile_step = gridDim.x;
 
     if (warp == 0 && lane == 0) {
         tma_prefetch_desc(&tmA);
@@ -128,7 +122,7 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
         }
         for (int a = 0; a < 2; ++a) {
             mbar_init(&acc_full[a], 1);
-            mbar_init(&acc_empty[a], EPI_WARPS * NCTA);   // one arrive per epilogue warp (of both CTAs of a pair)
+            mbar_init(&acc_empty[a], EPI_WARPS);          // one arrive per epilogue warp
         }
         for (int a = 0; a < 2 * EPI_WARPS; ++a) mbar_init(&res_bar[a], 1);
         if (p.tma_epi) {
@@ -137,13 +131,9 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
         }
         fence_mbar_init();
     }
-    if (warp == 1) {
-        if (NCTA == 2) tmem_alloc_pair<TMEM_COLS>(tmem_slot);
-        else tmem_alloc<TMEM_COLS>(tmem_slot);
-    }
+    if (warp == 1) tmem_alloc<TMEM_COLS>(tmem_slot);
     tc_fence_before();
-    if (NCTA == 2) cluster_sync_all();
-    else __syncthreads();
+    __syncthreads();
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
 
@@ -154,50 +144,32 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
             TileWalk tw(tile0, tile_step, tiles_m, tiles_n);
             for (int t = tile0; t < total_tiles; t += tile_step, tw.advance()) {
                 const int split = tw.split;
-                const int m0 = tw.m * BM_TILE + rank * BM, n0 = tw.n * BN + rank * BN_CTA;
+                const int m0 = tw.m * BM, n0 = tw.n * BN;
                 const int kb0 = split * p.kb_per_split, kb1 = min(total_kb, kb0 + p.kb_per_split);
                 for (int kb = kb0; kb < kb1; ++kb) {
                     mbar_wait(&empty_bar[s], phase ^ 1);
                     uint8_t* sA = smem + s * STAGE_BYTES;
                     uint8_t* sB = sA + A_STAGE_BYTES;
-                    if (NCTA == 2) {
-                        // the leader arms its barrier for the bytes of BOTH CTAs; either CTA's TMA completes on it
-                        if (rank == 0) mbar_arrive_expect_tx(&full_bar[s], 2 * STAGE_BYTES);
-                        const uint32_t bar = smem_u32(&full_bar[s]) & 0xFEFFFFFFu;      // same offset in the even CTA of the pair
-                        if (A_MN) {
+                    mbar_arrive_expect_tx(&full_bar[s], STAGE_BYTES);
+                    if (A_MN) {
 #pragma unroll
-                            for (int h = 0; h < BM / 64; ++h) tma_load_2d_pair(sA + h * (BK * 128), &tmA, bar, m0 + h * 64, kb * BK);
-                        } else {
-                            tma_load_2d_pair(sA, &tmA, bar, kb * BK, m0);
-                        }
-                        if (B_MN) {
-#pragma unroll
-                            for (int h = 0; h < BN_CTA / 64; ++h) tma_load_2d_pair(sB + h * (BK * 128), &tmB, bar, n0 + h * 64, kb * BK);
-                        } else {
-                            tma_load_2d_pair(sB, &tmB, bar, kb * BK, n0);
-                        }
+                        for (int h = 0; h < BM / 64; ++h) tma_load_2d(sA + h * (BK * 128), &tmA, &full_bar[s], m0 + h * 64, kb * BK);
                     } else {
-                        mbar_arrive_expect_tx(&full_bar[s], STAGE_BYTES);
-                        if (A_MN) {
+                        tma_load_2d(sA, &tmA, &full_bar[s], kb * BK, m0);
+                    }
+                    if (B_MN) {
 #pragma unroll
-                            for (int h = 0; h < BM / 64; ++h) tma_load_2d(sA + h * (BK * 128), &tmA, &full_bar[s], m0 + h * 64, kb * BK);
-                        } else {
-                            tma_load_2d(sA, &tmA, &full_bar[s], kb * BK, m0);
-                        }
-                        if (B_MN) {
-#pragma unroll
-                            for (int h = 0; h < BN / 64; ++h) tma_load_2d(sB + h * (BK * 128), &tmB, &full_bar[s], n0 + h * 64, kb * BK);
-                        } else {
-                            tma_load_2d(sB, &tmB, &full_bar[s], kb * BK, n0);
-                        }
+                        for (int h = 0; h < BN / 64; ++h) tma_load_2d(sB + h * (BK * 128), &tmB, &full_bar[s], n0 + h * 64, kb * BK);
+                    } else {
+                        tma_load_2d(sB, &tmB, &full_bar[s], kb * BK, n0);
                     }
                     if (++s == STAGES) { s = 0; phase ^= 1; }
                 }
             }
         }
     } else if (warp == 1) {
-        if (lane == 0 && rank == 0) {
-            constexpr uint32_t idesc = umma_idesc_bf16(BM_TILE, BN, A_MN, B_MN);
+        if (lane == 0) {
+            constexpr uint32_t idesc = umma_idesc_bf16(BM, BN, A_MN, B_MN);
             // K-major: 8-row groups are 1024 B apart (SBO); LBO unused.  MN-major: 64-element MN atoms
             // are BK*128 B apart (LBO), 8-k-row groups 1024 B apart (SBO).
             constexpr uint32_t a_lbo = A_MN ? BK * 128 : 0, b_lbo = B_MN ? BK * 128 : 0;
@@ -209,7 +181,7 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
             for (int t = tile0; t < total_tiles; t += tile_step, tw.advance()) {
                 const int split = tw.split;
                 const int kb0 = split * p.kb_per_split, kb1 = min(total_kb, kb0 + p.kb_per_split);
-                mbar_wait(&acc_empty[acc], acc_phase ^ 1);       // epilogue (of both CTAs) has drained this accumulator buffer
+                mbar_wait(&acc_empty[acc], acc_phase ^ 1);       // epilogue has drained this accumulator buffer
                 tc_fence_after();
                 const uint32_t tmem_d = tmem_base + (uint32_t)(acc * BN);
                 for (int i = 0; i < kb1 - kb0; ++i) {
@@ -221,15 +193,12 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
                     for (int k = 0; k < BK / UMMA_K; ++k) {
                         const uint64_t da = umma_smem_desc_sw128(a_addr + k * a_kstep, a_lbo, 1024);
                         const uint64_t db = umma_smem_desc_sw128(b_addr + k * b_kstep, b_lbo, 1024);
-                        if (NCTA == 2) umma_bf16_pair(tmem_d, da, db, idesc, (i > 0 || k > 0) ? 1u : 0u);
-                        else umma_bf16(tmem_d, da, db, idesc, (i > 0 || k > 0) ? 1u : 0u);
+                        umma_bf16(tmem_d, da, db, idesc, (i > 0 || k > 0) ? 1u : 0u);
                     }
-                    if (NCTA == 2) umma_commit_pair(&empty_bar[s]);      // frees the stage in both CTAs
-                    else umma_commit(&empty_bar[s]);
+                    umma_commit(&empty_bar[s]);
                     if (++s == STAGES) { s = 0; phase ^= 1; }
                 }
-                if (NCTA == 2) umma_commit_pair(&acc_full[acc]);
-                else umma_commit(&acc_full[acc]);
+                umma_commit(&acc_full[acc]);
                 if (++acc == 2) { acc = 0; acc_phase ^= 1; }
             }
         }
@@ -239,11 +208,6 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
         const int q = warp & 3;
         const int ew = warp - 2;
         const float alpha = p.alpha != nullptr ? __ldg(p.alpha) : 1.f;
-        const uint32_t acc_empty_leader[2] = {NCTA == 2 ? mapa_u32(&acc_empty[0], 0) : 0u, NCTA == 2 ? mapa_u32(&acc_empty[1], 0) : 0u};
-        auto release_acc = [&](int a) {
-            if (NCTA == 2) mbar_arrive_cluster(acc_empty_leader[a]);
-            else mbar_arrive(&acc_empty[a]);
-        };
         if (p.tma_epi) {
             // TMA epilogue.  Unit of work = one 4 KB box of C: 32 rows x 128 bytes (64 bf16 or 32 fp32 columns).  Each thread
             // converts its own row straight out of TMEM (+alpha, bias, rowmask, residual), writes it into a 128B-swizzled
@@ -278,7 +242,7 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
             TileWalk tw(tile0, tile_step, tiles_m, tiles_n);
             fetch_bias(tile0, tw.n);
             for (int t = tile0; t < total_tiles; t += tile_step) {
-                const int m0 = tw.m * BM_TILE + rank * BM, n0 = tw.n * BN;
+                const int m0 = tw.m * BM, n0 = tw.n * BN;
                 tw.advance();                        // tw now describes the NEXT tile of this CTA (bias prefetch below)
                 const int row_base = m0 + q * 32;
                 const int row = row_base + lane;
@@ -298,7 +262,7 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
                     // nothing of this tile belongs to this warp: hand the accumulator back at once
                     tc_fence_before();
                     __syncwarp();
-                    if (lane == 0) release_acc(acc);
+                    if (lane == 0) mbar_arrive(&acc_empty[acc]);
                     last_u = -1;
                 }
 #pragma unroll 1
@@ -320,7 +284,7 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
                         if (u == last_u) {
                             tc_fence_before();
                             __syncwarp();
-                            if (lane == 0) release_acc(acc);
+                            if (lane == 0) mbar_arrive(&acc_empty[acc]);
                         }
                         if (p.residual != nullptr) {
                             mbar_wait(&rbar[ubuf], (rphase >> ubuf) & 1u);
@@ -351,7 +315,7 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
                         if (u == last_u) {
                             tc_fence_before();
                             __syncwarp();
-                            if (lane == 0) release_acc(acc);
+                            if (lane == 0) mbar_arrive(&acc_empty[acc]);
                         }
                         if (p.rowdot_out != nullptr) {
                             mbar_wait(&rbar[ubuf], (rphase >> ubuf) & 1u);
@@ -421,7 +385,7 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
             uint32_t acc_phase = 0;
             for (int t = tile0; t < total_tiles; t += tile_step) {
                 const int rem = t % tiles_mn;      // (fallback path: keeps the plain decode)
-                const int m0 = (rem / tiles_n) * BM_TILE + rank * BM, n0 = (rem % tiles_n) * BN;
+                const int m0 = (rem / tiles_n) * BM, n0 = (rem % tiles_n) * BN;
                 const int row_base = m0 + q * 32;
                 mbar_wait(&acc_full[acc], acc_phase);
                 tc_fence_after();
@@ -448,7 +412,7 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
                         released = true;
                         tc_fence_before();
                         __syncwarp();
-                        if (lane == 0) release_acc(acc);
+                        if (lane == 0) mbar_arrive(&acc_empty[acc]);
                     }
                     if (!live) break;
                     __syncwarp();
@@ -510,13 +474,8 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
     }
     __syncwarp();
     tc_fence_before();
-    if (NCTA == 2) {
-        cluster_sync_all();          // the peer's smem / barriers must outlive the leader's last MMA and commit
-        if (warp == 1) tmem_dealloc_pair<TMEM_COLS>(tmem_base);
-    } else {
-        __syncthreads();
-        if (warp == 1) tmem_dealloc<TMEM_COLS>(tmem_base);
-    }
+    __syncthreads();
+    if (warp == 1) tmem_dealloc<TMEM_COLS>(tmem_base);
 }
 
 typedef CUresult (*PFN_encodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
@@ -535,31 +494,18 @@ PFN_encodeTiled get_encode_fn() {
     return fn;
 }
 
-template <int BN, bool A_MN, bool B_MN, int NCTA>
+template <int BN, bool A_MN, bool B_MN>
 int launch_gemm(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmC, const CUtensorMap& tmR, const GemmParams& p,
                 int splits, cudaStream_t stream) {
-    auto kern = gemm_bf16_kernel<BN, A_MN, B_MN, NCTA>;
+    auto kern = gemm_bf16_kernel<BN, A_MN, B_MN>;
     static bool configured = false;
     if (!configured) {
-        SPB_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, gemm_smem_bytes<BN, NCTA>()));
+        SPB_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, gemm_smem_bytes<BN>()));
         configured = true;
     }
-    const int total_tiles = ceil_div(p.N, BN) * ceil_div(p.M, BM * NCTA) * splits;
-    const int max_units = spb_num_sms() / NCTA;                       // one CTA (pair) per SM (pair)
-    const int grid = (total_tiles < max_units ? total_tiles : max_units) * NCTA;
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(grid);
-    cfg.blockDim = dim3(GEMM_THREADS);
-    cfg.dynamicSmemBytes = gemm_smem_bytes<BN, NCTA>();
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = NCTA;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    SPB_CHECK_CUDA(cudaLaunchKernelEx(&cfg, kern, tmA, tmB, tmC, tmR, p));
+    const int total_tiles = ceil_div(p.N, BN) * ceil_div(p.M, BM) * splits;
+    const int grid = total_tiles < spb_num_sms() ? total_tiles : spb_num_sms();      // one CTA per SM
+    kern<<<grid, GEMM_THREADS, gemm_smem_bytes<BN>(), stream>>>(tmA, tmB, tmC, tmR, p);
     SPB_CHECK_LAUNCH();
     return SPB_OK;
 }
@@ -643,23 +589,17 @@ static int gemm_impl(const void* A, const void* B, void* C, int M, int N, int K,
     SPB_CHECK_ARG(!(accumulate || split_k > 1) || c_fp32, "spb_gemm_bf16: split-K / accumulate need an fp32 C");
 
     int BN = (N <= 64) ? 64 : 128;
-    // CTA pairs (256-row tiles, each CTA staging half of B) and wide tiles cut the L2->SM operand traffic per output.
-    // SPB_GEMM_BN / SPB_GEMM_NCTA / SPB_GEMM_EPI override the heuristics for experiments.
-    int ncta = 1;
-    if (const char* e = getenv("SPB_GEMM_NCTA")) { int v = atoi(e); if (v == 1 || (v == 2 && N > 64 && M > BM)) ncta = v; }
-    if (ncta == 2) { if (N % 256 == 0 && M >= 8 * BM) BN = 256; }
-    else if (N % 256 == 0 && M >= 8 * BM) BN = 256;
-    if (const char* e = getenv("SPB_GEMM_BN")) { int v = atoi(e); if ((v == 64 && ncta == 1) || v == 128 || v == 256) BN = v; }
+    // wide tiles cut the L2->SM operand traffic per output.  SPB_GEMM_BN / SPB_GEMM_EPI override the heuristics for experiments.
+    if (N % 256 == 0 && M >= 8 * BM) BN = 256;
+    if (const char* e = getenv("SPB_GEMM_BN")) { int v = atoi(e); if (v == 64 || v == 128 || v == 256) BN = v; }
     const int total_kb = ceil_div(K, BK);
     int splits = 1;
     if (split_k > 1) splits = split_k;
     else if (split_k == 0 && c_fp32 && bias == nullptr && residual == nullptr && rowmask == nullptr) {
         // auto split-K for tall-K / small-output problems (wgrad)
-        const int tiles = ceil_div(M, BM * ncta) * ceil_div(N, BN);
-        int mult = 1;      // one work item per SM measured best (fewer partial tiles to reduce-add into the same lines)
-        if (const char* e = getenv("SPB_GEMM_SPLIT_MULT")) { int v = atoi(e); if (v >= 1 && v <= 8) mult = v; }
-        const int units = spb_num_sms() / ncta, target = mult * units;
-        if (tiles < units && total_kb >= 8) splits = max(1, min(total_kb / 4, target / tiles));
+        // one work item per SM measured best (fewer partial tiles to reduce-add into the same lines)
+        const int tiles = ceil_div(M, BM) * ceil_div(N, BN), units = spb_num_sms();
+        if (tiles < units && total_kb >= 8) splits = max(1, min(total_kb / 4, units / tiles));
     }
     int kb_per_split = ceil_div(total_kb, splits);
     splits = ceil_div(total_kb, kb_per_split);
@@ -670,7 +610,7 @@ static int gemm_impl(const void* A, const void* B, void* C, int M, int N, int K,
     else rc = spb_make_tmap_bf16_2d(&tmA, A, (uint64_t)K, (uint64_t)M, (uint64_t)lda * 2, BK, BM);
     if (rc != SPB_OK) return rc;
     if (trans_b) rc = spb_make_tmap_bf16_2d(&tmB, B, (uint64_t)N, (uint64_t)K, (uint64_t)ldb * 2, 64, BK);
-    else rc = spb_make_tmap_bf16_2d(&tmB, B, (uint64_t)K, (uint64_t)N, (uint64_t)ldb * 2, BK, (uint32_t)(BN / ncta));
+    else rc = spb_make_tmap_bf16_2d(&tmB, B, (uint64_t)K, (uint64_t)N, (uint64_t)ldb * 2, BK, (uint32_t)BN);
     if (rc != SPB_OK) return rc;
 
     // TMA epilogue whenever C (and the residual) satisfy the 16-byte base / row-pitch rules of a tensor map
@@ -716,18 +656,14 @@ static int gemm_impl(const void* A, const void* B, void* C, int M, int N, int K,
         else SPB_CHECK_CUDA(cudaMemset2DAsync(C, (size_t)ldc * 4, 0, (size_t)N * 4, M, stream));
     }
 
-#define SPB_DISPATCH(BN_, NCTA_)                                                                                     \
-    if (trans_a && trans_b) return launch_gemm<BN_, true, true, NCTA_>(tmA, tmB, tmC, tmR, p, splits, stream);      \
-    if (trans_a) return launch_gemm<BN_, true, false, NCTA_>(tmA, tmB, tmC, tmR, p, splits, stream);                \
-    if (trans_b) return launch_gemm<BN_, false, true, NCTA_>(tmA, tmB, tmC, tmR, p, splits, stream);                \
-    return launch_gemm<BN_, false, false, NCTA_>(tmA, tmB, tmC, tmR, p, splits, stream);
-    if (ncta == 2) {
-        if (BN == 256) { SPB_DISPATCH(256, 2) }
-        SPB_DISPATCH(128, 2)
-    }
-    if (BN == 64) { SPB_DISPATCH(64, 1) }
-    if (BN == 256) { SPB_DISPATCH(256, 1) }
-    SPB_DISPATCH(128, 1)
+#define SPB_DISPATCH(BN_)                                                                                     \
+    if (trans_a && trans_b) return launch_gemm<BN_, true, true>(tmA, tmB, tmC, tmR, p, splits, stream);      \
+    if (trans_a) return launch_gemm<BN_, true, false>(tmA, tmB, tmC, tmR, p, splits, stream);                \
+    if (trans_b) return launch_gemm<BN_, false, true>(tmA, tmB, tmC, tmR, p, splits, stream);                \
+    return launch_gemm<BN_, false, false>(tmA, tmB, tmC, tmR, p, splits, stream);
+    if (BN == 64) { SPB_DISPATCH(64) }
+    if (BN == 256) { SPB_DISPATCH(256) }
+    SPB_DISPATCH(128)
 #undef SPB_DISPATCH
 }
 

@@ -11,8 +11,6 @@
 // one fp32 atomic per column per CTA.
 #include "common.cuh"
 
-#include <stdlib.h>
-
 namespace {
 
 constexpr int ROW_WARPS = 8;
@@ -404,61 +402,6 @@ embed_ln_bwd_stats_kernel(const __nv_bfloat16* __restrict__ dy, int ld_dy, const
     }
 }
 
-// Backward pass 2: grid (chunks, F).  The CTA privatises field f's table gradient [V_f, 128] in shared memory,
-// scatters dx = rstd * (dy*w - c1 - xhat*c2) for its chunk of tuples with shared-memory atomics, then flushes
-// once.  PAD (token 0) rows receive no gradient (F.embedding padding_idx=0, modules/transformer/embeddings.py:99).
-constexpr int SCATTER_WARPS = 16;
-__global__ void __launch_bounds__(SCATTER_WARPS * 32)
-embed_ln_bwd_scatter_kernel(const __nv_bfloat16* __restrict__ dy, int ld_dy, const int64_t* __restrict__ tokens, int ld_tok,
-                            const float* __restrict__ table, FieldTable ft, const float* __restrict__ w,
-                            const float* __restrict__ mean_in, const float* __restrict__ rstd_in,
-                            const float* __restrict__ c1_in, const float* __restrict__ c2_in, float* __restrict__ dtable,
-                            int n_rows, int rows_per_chunk) {
-    extern __shared__ float stab[];
-    const int f = blockIdx.y;
-    const int V = ft.size[f], off = ft.offset[f];
-    for (int i = threadIdx.x; i < V * 128; i += blockDim.x) stab[i] = 0.f;
-    __syncthreads();
-    const int lane = threadIdx.x & 31;
-    const int warp = threadIdx.x >> 5;
-    const int r0 = blockIdx.x * rows_per_chunk;
-    const int r1 = min(n_rows, r0 + rows_per_chunk);
-    const int c = f * 128 + lane * 4;
-    const float4 g = *reinterpret_cast<const float4*>(w + c);
-    constexpr int U = 4;   // tuples in flight per warp: the loop is latency-bound (gather -> shared atomic), so batch the loads
-    for (int base = r0 + warp * U; base < r1; base += SCATTER_WARPS * U) {
-        long long tok[U];
-        float4 xv[U];
-        uint2 dv[U];
-        float st[U][4];
-#pragma unroll
-        for (int u = 0; u < U; ++u) {
-            const int row = base + u;
-            tok[u] = row < r1 ? tokens[(size_t)row * ld_tok + f] : 0;
-            if (tok[u] <= 0 || tok[u] >= V) { tok[u] = 0; continue; }   // PAD / out of range: no gradient
-            xv[u] = *reinterpret_cast<const float4*>(table + (size_t)(off + tok[u]) * 128 + lane * 4);
-            dv[u] = *reinterpret_cast<const uint2*>(dy + (size_t)row * ld_dy + c);
-            st[u][0] = mean_in[row]; st[u][1] = rstd_in[row]; st[u][2] = c1_in[row]; st[u][3] = c2_in[row];
-        }
-#pragma unroll
-        for (int u = 0; u < U; ++u) {
-            if (tok[u] == 0) continue;
-            const float mean = st[u][0], rstd = st[u][1], c1 = st[u][2], c2 = st[u][3];
-            const float2 d0 = unpack_bf16x2(dv[u].x), d1 = unpack_bf16x2(dv[u].y);
-            float* dst = stab + (size_t)tok[u] * 128 + lane * 4;
-            atomicAdd(dst + 0, rstd * (d0.x * g.x - c1 - (xv[u].x - mean) * rstd * c2));
-            atomicAdd(dst + 1, rstd * (d0.y * g.y - c1 - (xv[u].y - mean) * rstd * c2));
-            atomicAdd(dst + 2, rstd * (d1.x * g.z - c1 - (xv[u].z - mean) * rstd * c2));
-            atomicAdd(dst + 3, rstd * (d1.y * g.w - c1 - (xv[u].w - mean) * rstd * c2));
-        }
-    }
-    __syncthreads();
-    for (int i = threadIdx.x; i < V * 128; i += blockDim.x) {
-        const float v = stab[i];
-        if (v != 0.f) atomicAdd(dtable + (size_t)off * 128 + i, v);
-    }
-}
-
 int row_grid(int n_rows) {
     int blocks = ceil_div(n_rows, ROW_WARPS);
     int cap = spb_num_sms() * 8;
@@ -627,23 +570,5 @@ extern "C" int spb_embed_ln_bwd(const void* dy, int ld_dy, const int64_t* tokens
         return SPB_ERR_ARG;
     }
     SPB_CHECK_LAUNCH();
-    if (getenv("SPB_EMBED_SCATTER_ATOMIC") == nullptr)
-        return spb_embed_scatter_mma(d, ld_dy, tokens, ld_tok, table, ft, w, mean, rstd, c1, c2, dtable, n_rows, stream);
-    int max_v = 0;
-    for (int f = 0; f < n_fields; ++f) max_v = field_sizes[f] > max_v ? field_sizes[f] : max_v;
-    const size_t smem = (size_t)max_v * 128 * sizeof(float);
-    SPB_CHECK_ARG(smem <= 220 * 1024, "spb_embed_ln_bwd: field vocabulary %d too large for the shared-memory scatter", max_v);
-    static size_t configured = 0;
-    if (smem > configured) {
-        SPB_CHECK_CUDA(cudaFuncSetAttribute(embed_ln_bwd_scatter_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        configured = smem;
-    }
-    int chunks = ceil_div(2 * spb_num_sms(), n_fields);
-    int rows_per_chunk = ceil_div(n_rows, chunks);
-    if (rows_per_chunk < 64) rows_per_chunk = 64;
-    chunks = ceil_div(n_rows, rows_per_chunk);
-    embed_ln_bwd_scatter_kernel<<<dim3(chunks, n_fields), SCATTER_WARPS * 32, smem, stream>>>(d, ld_dy, tokens, ld_tok, table, ft, w, mean, rstd,
-                                                                              c1, c2, dtable, n_rows, rows_per_chunk);
-    SPB_CHECK_LAUNCH();
-    return SPB_OK;
+    return spb_embed_scatter_mma(d, ld_dy, tokens, ld_tok, table, ft, w, mean, rstd, c1, c2, dtable, n_rows, stream);
 }

@@ -246,7 +246,7 @@ def render_decoder(dec, perf: Tensor, masked_perf: Tensor, score_hidden: Tensor,
     # Everything of a note-step that does not depend on the tokens sampled so far is evaluated for ALL positions before the loop,
     # in large launches: the masked tuple of note i+1 through the embedding and its half of project_multiemb (+ bias), and the
     # context half of project_emb (+ bias).  A step then adds its own half (the previous, complete tuple) as a GEMM with a residual.
-    lean = plan is not None and K._os.environ.get("SPB_DECODE_FRONT", "lean") == "lean"
+    lean = plan is not None
     if lean:
         Dm = dec.dim
         wm_r, wc_l, wc_r = wm16[:, Dm:], wc16[:, :Dm], wc16[:, Dm:]

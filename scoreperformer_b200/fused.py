@@ -10,14 +10,10 @@ from __future__ import annotations
 from dataclasses import dataclass
 from typing import List, Optional, Sequence, Tuple
 
-import contextlib
-import os
-
 import torch
 from torch import Tensor
 
 from . import kernels as K
-from .utils import SideBranch
 
 BF16, F32 = torch.bfloat16, torch.float32
 
@@ -29,9 +25,8 @@ BF16, F32 = torch.bfloat16, torch.float32
 DIRECT_GRAD = False
 SHADOW_ACTIVE = False
 # STACK_BACKWARD_DONE: callable(params) or None.  TransformerStackFn.backward calls it once every weight gradient of its stack has
-#   been written (and the weight-gradient side streams have been joined): TrainStep launches that stack's gradient bucket on NCCL.
+#   been written: TrainStep launches that stack's gradient bucket on NCCL.
 STACK_BACKWARD_DONE = None
-HEAD_PROJ_FP32 = os.environ.get("SPB_HEAD_PROJ", "fp32") == "fp32"
 
 
 def _shadow(param: Tensor) -> Optional[Tensor]:
@@ -430,16 +425,6 @@ class TransformerStackFn(torch.autograd.Function):
             grads[j], grads[j + 1] = (None if d1 else dw), (None if d2 else db)
             return res if want16 else (res, None)
 
-        # weight-gradient GEMMs feed nothing downstream in this backward, so they CAN run on a side stream of their own (one per
-        # calling stream), joined before the gradients are handed to autograd.  Off by default since round 2: every large kernel
-        # of the chain is persistent and owns all SMs, so the branch only delays the chain (measured 10.54 vs 10.16 ms per C2 step)
-        wb = None
-        if g_out.is_cuda and os.environ.get("SPB_WGRAD_BRANCH", "0") == "1":
-            for i in range(3):                                     # small fixed pool, created on the first (eager) call
-                SideBranch(g_out.device, slot=("wgrad", i))
-            wb = SideBranch(g_out.device, slot=("wgrad", (torch.cuda.current_stream().cuda_stream >> 6) % 3))
-        side = (lambda *ts: wb.run(*ts)) if wb is not None else (lambda *ts: contextlib.nullcontext())
-
         g, g16 = norm_bwd(2 * spec.depth, K.cast_bf16(g_out.contiguous().view(N, D)), ctx.final, None)
         w2t_all = None
         if K.ffn_bwd_fused_ok(D, spec.ff_inner):       # out-projection weights of every layer, transposed in one launch
@@ -449,8 +434,7 @@ class TransformerStackFn(torch.autograd.Function):
             rec_a, rec_f = ctx.layers[l]
             # ---- feed-forward backward:  x_out = x + W2 glu(W1 LN(x) + b1)
             p_w1, p_b1, p_w2 = params[base + PARAMS_PER_ATTN + 2:base + PARAMS_PER_ATTN + 5]
-            with side(g16, rec_f["h"]):
-                grads[base + PARAMS_PER_ATTN + 4] = wgrad(p_w2, g16, rec_f["h"])
+            grads[base + PARAMS_PER_ATTN + 4] = wgrad(p_w2, g16, rec_f["h"])
             db1, d_b1 = take(p_b1)
             if K.ffn_bwd_fused_ok(D, spec.ff_inner):
                 # one kernel: dh = dy W2 (on chip) -> GLU' . mask -> du (written over u) -> dxn = du W1, db1 += colsum(du)
@@ -464,15 +448,13 @@ class TransformerStackFn(torch.autograd.Function):
                 du = K.glu_bwd(dh, rec_f["u"], db1, p_ff, ctx.seeds[2 * l + 1])
                 dxn = None
             grads[base + PARAMS_PER_ATTN + 3] = None if d_b1 else db1
-            with side(du, rec_f["xn"]):
-                grads[base + PARAMS_PER_ATTN + 2] = wgrad(p_w1, du, rec_f["xn"])
+            grads[base + PARAMS_PER_ATTN + 2] = wgrad(p_w1, du, rec_f["xn"])
             if dxn is None:
                 dxn = K.gemm(du, rec_f["w1_16"], trans_b=True, out_dtype=BF16)
             g, g16 = norm_bwd(2 * l + 1, dxn, rec_f, g)
             # ---- attention backward:  x_out = x + mask * Wo attn(Wqkv LN(x))
             p_q, p_k, p_v, p_o, p_ls = params[base + 2:base + 7]
-            with side(g16, rec_a["o"]):
-                grads[base + 5] = wgrad(p_o, g16, rec_a["o"])
+            grads[base + 5] = wgrad(p_o, g16, rec_a["o"])
             # dO = dY Wo and delta = rowsum(dO * O) in one GEMM (the epilogue owns whole rows of a head)
             do, delta = K.gemm_rowdot(g16, rec_a["wo16"], rec_a["o"], T, H, trans_b=True)
             dls, d_ls = take(p_ls)
@@ -480,13 +462,12 @@ class TransformerStackFn(torch.autograd.Function):
                                    ctx.seeds[2 * l], delta=delta, aux=rec_a["aux"])
             grads[base + 6] = None if d_ls else dls.view(p_ls.shape)
             g_qkv = direct_grad_cat([p_q, p_k, p_v])
-            with side(dqkv, rec_a["xn"]):
-                if g_qkv is not None:
-                    K.gemm(dqkv, rec_a["xn"], trans_a=True, trans_b=True, out=g_qkv, split_k=0, accumulate=True)
-                else:
-                    dwqkv = K.gemm(dqkv, rec_a["xn"], trans_a=True, trans_b=True, out_dtype=F32, split_k=0)
-                    hq = H * spec.dim_head
-                    grads[base + 2], grads[base + 3], grads[base + 4] = dwqkv[:hq], dwqkv[hq:hq + spec.dim_head], dwqkv[hq + spec.dim_head:]
+            if g_qkv is not None:
+                K.gemm(dqkv, rec_a["xn"], trans_a=True, trans_b=True, out=g_qkv, split_k=0, accumulate=True)
+            else:
+                dwqkv = K.gemm(dqkv, rec_a["xn"], trans_a=True, trans_b=True, out_dtype=F32, split_k=0)
+                hq = H * spec.dim_head
+                grads[base + 2], grads[base + 3], grads[base + 4] = dwqkv[:hq], dwqkv[hq:hq + spec.dim_head], dwqkv[hq + spec.dim_head:]
             dxn = K.gemm(dqkv, rec_a["wqkv16"], trans_b=True, out_dtype=BF16)
             g, g16 = norm_bwd(2 * l, dxn, rec_a, g)
         d_style = None
@@ -508,8 +489,6 @@ class TransformerStackFn(torch.autograd.Function):
             K.multi_add(add_dst, add_src)
             if ctx.needs_input_grad[3]:
                 d_style = K.gemm(dgb_all, w_ada16, trans_b=True, out_dtype=F32).view(ctx.style_shape)
-        if wb is not None:
-            wb.join(*[t for t in grads if isinstance(t, Tensor)])
         if STACK_BACKWARD_DONE is not None and DIRECT_GRAD:
             STACK_BACKWARD_DONE(params)
         return (None, g.view(B, T, D), None, d_style, None) + tuple(grads)
@@ -638,7 +617,7 @@ class TiedHeadCEFn(torch.autograd.Function):
         h16 = K.cast_bf16(hidden.contiguous()) if hidden.dtype == F32 else hidden.contiguous()
         wp16 = w16(proj_w)                                          # [dim, F*emb]
         # the projection stays fp32 until its LayerNorm (one bf16 rounding less in front of the logits; 1536 columns only)
-        e_raw = K.gemm(h16, wp16, trans_b=True, out_dtype=F32 if HEAD_PROJ_FP32 else BF16)     # [n, F*emb]
+        e_raw = K.gemm(h16, wp16, trans_b=True, out_dtype=F32)     # [n, F*emb]
         e, mean, rstd = K.layer_norm_fwd(e_raw, ln_w, ln_b, out_dtype=BF16)
         table16 = K.cast_bf16(table.contiguous())
         offs = [0]
@@ -766,7 +745,7 @@ def tied_head_logits(hidden: Tensor, proj_w: Tensor, ln_w: Tensor, ln_b: Tensor,
     """Inference-side logits (fp32 [n, V_f] per requested field); no autograd."""
     with torch.no_grad():
         h16 = K.cast_bf16(hidden.contiguous()) if hidden.dtype == F32 else hidden.contiguous()
-        e_raw = K.gemm(h16, K.cast_bf16(proj_w.contiguous()), trans_b=True, out_dtype=F32 if HEAD_PROJ_FP32 else BF16)
+        e_raw = K.gemm(h16, K.cast_bf16(proj_w.contiguous()), trans_b=True, out_dtype=F32)
         e, _, _ = K.layer_norm_fwd(e_raw, ln_w, ln_b, out_dtype=BF16, need_stats=False)
         table16 = K.cast_bf16(table.contiguous())
         offs = [0]

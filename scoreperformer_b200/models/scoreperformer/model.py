@@ -217,7 +217,7 @@ class ScorePerformer(_LMMixin, Model):
         # the decoder's input embedding needs the score embeddings but not the latents: it runs behind the score encoder, next to
         # the performance encoder, instead of after both
         pre_embed = None
-        if self.score_encoder is not None and hasattr(self.perf_decoder, "pre_embed") and _os.environ.get("SPB_DEC_PRE_EMBED", "1") == "1":
+        if self.score_encoder is not None and hasattr(self.perf_decoder, "pre_embed"):
             pre_embed = lambda score_emb: self.perf_decoder.pre_embed(perf, masked_perf, score_emb, table_cache)
         enc_out = self.forward_encoders(
             perf=default(noisy_perf, perf), perf_mask=default(noisy_perf_mask, perf_mask), score=score, score_mask=score_mask,

@@ -134,9 +134,6 @@ class TrainStep:
             self._next_bucket += 1
 
     def _all_reduce(self, t: Tensor):
-        if os.environ.get("SPB_DDP_SYNCOPS", "0") == "1":
-            dist.all_reduce(t, op=dist.ReduceOp.SUM, group=self.group)
-            return None
         return dist.all_reduce(t, op=dist.ReduceOp.SUM, group=self.group, async_op=True)
 
     def _forward_backward(self, batch: Dict[str, Tensor]):
@@ -171,8 +168,7 @@ class TrainStep:
                     self._works.append(self._all_reduce(self.flat_grad[pos:lo]))
                 pos = max(pos, hi)
             for w in self._works:
-                if w is not None:
-                    w.wait()
+                w.wait()
             self._works = []
         norm = torch.linalg.vector_norm(self.flat_grad) if self.grad_clip is not None else None
         self.opt_step.add_(1)

@@ -2,7 +2,6 @@ import sys, time, torch
 sys.path.insert(0, ".")
 from tests import parity
 from scoreperformer_b200 import decode
-from scoreperformer_b200 import kernels as K
 model = parity.build_model(dropout=False, device="cuda").eval()
 B, T = 256, 1024
 batch = {k: v.cuda() for k, v in parity.make_batch(B, T, seed=5, full_length=True, deadpan_last=False).items()}
@@ -25,4 +24,4 @@ with torch.inference_mode():
         torch.cuda.synchronize(); t0 = time.perf_counter()
         out = decode.render_batch(model, tokens, batch["masked_perf"], enc.score_embeddings, enc.perf_embeddings, mask=batch["perf_mask"])
         torch.cuda.synchronize(); t1 = time.perf_counter()
-        print(f"{K._os.environ.get('SPB_DECODE_FRONT', 'lean')} rep {rep}: total {t1 - t0:.3f} s; before first replay {marks['first_replay'] - t0:.3f} s; replays {t1 - marks['first_replay']:.3f} s")
+        print(f"rep {rep}: total {t1 - t0:.3f} s; before first replay {marks['first_replay'] - t0:.3f} s; replays {t1 - marks['first_replay']:.3f} s")

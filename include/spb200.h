@@ -202,7 +202,9 @@ int spb_attention_bwd(const void* qkv, int ld, const uint8_t* key_mask, const fl
 /* KV-cached incremental decode (one new query per sequence): q bf16 [B, H*64]; kv cache bf16 rows of (k | v); the query sits at
  * position q_pos.  Replaces the cached path of attention.py:155-156 / transformer.py:161-186 without the per-step torch.cat.
  * pos_dev (optional): device int64 holding q_pos -- n_keys is then the cache capacity, which makes the launch replayable from a
- * CUDA graph; append_kv: first copy columns [H*64, H*64+128) of every q row (the new k | v) into cache row q_pos. */
+ * CUDA graph; append_kv: first copy columns [H*64, H*64+128) of every q row (the new k | v) into cache row q_pos (nothing when a
+ * device position is outside the cache; a host q_pos outside [0, n_keys) is rejected).  Returns -1 when the H * n_keys fp32 scores
+ * exceed the device's shared memory per block. */
 int spb_attention_decode(const void* q, int ld_q, void* kv, int ld_kv, long long kv_batch_stride, const uint8_t* key_mask,
                          int mask_stride, const float* logslopes, void* out, int ld_out, int B, int H, int dim_head, int n_keys,
                          int q_pos, const int64_t* pos_dev, int append_kv, spb_stream_t stream);

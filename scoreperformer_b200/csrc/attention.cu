@@ -706,8 +706,9 @@ __global__ void attn_decode_kernel(const __nv_bfloat16* __restrict__ q, int ld_q
     float* p = sp + (size_t)h * cap;
     __nv_bfloat16* kvb = const_cast<__nv_bfloat16*>(kv) + (size_t)b * kv_batch_stride;
     if (append_kv) {
-        // the new position's (k | v) sit right after the H query heads of this row: append them to the cache first
-        if (threadIdx.x < 16)
+        // the new position's (k | v) sit right after the H query heads of this row: append them to the cache first.  A device
+        // position is caller data that the host never sees: a row outside the cache is not written
+        if (threadIdx.x < 16 && q_pos >= 0 && q_pos < cap)
             reinterpret_cast<uint4*>(kvb + (size_t)q_pos * ld_kv)[threadIdx.x] =
                 reinterpret_cast<const uint4*>(q + (size_t)b * ld_q + n_heads * DH)[threadIdx.x];
         __syncthreads();
@@ -794,7 +795,8 @@ __global__ void attn_decode_kernel(const __nv_bfloat16* __restrict__ q, int ld_q
 // q bf16 [B, >= H*64] (row stride ld_q); kv bf16 cache [B][n_keys rows of (k | v) = 128 columns] (row stride ld_kv, batch stride in
 // elements); key_mask [B, mask_stride] or NULL; out bf16 [B, H*64].  The query sits at position q_pos (keys j <= q_pos attend).
 // pos_dev (optional): device int64 holding q_pos; n_keys is then the cache CAPACITY and keys j <= *pos_dev are used.
-// append_kv: copy columns [H*64, H*64+128) of each q row into cache row q_pos before attending (saves a separate copy).
+// append_kv: copy columns [H*64, H*64+128) of each q row into cache row q_pos before attending (saves a separate copy); a device
+// position outside [0, capacity) appends nothing.  H * n_keys fp32 scores must fit the device's shared memory per block.
 extern "C" int spb_attention_decode(const void* q, int ld_q, void* kv, int ld_kv, long long kv_batch_stride, const uint8_t* key_mask,
                                     int mask_stride, const float* logslopes, void* out, int ld_out, int B, int H, int dim_head,
                                     int n_keys, int q_pos, const int64_t* pos_dev, int append_kv, cudaStream_t stream) {
@@ -803,7 +805,17 @@ extern "C" int spb_attention_decode(const void* q, int ld_q, void* kv, int ld_kv
     SPB_CHECK_ARG(dim_head == DH && H >= 1 && H <= 32, "spb_attention_decode: dim_head must be %d, 1..32 heads", DH);
     SPB_CHECK_ARG(n_keys <= DEC_MAX_T, "spb_attention_decode: at most %d cached keys", DEC_MAX_T);
     SPB_CHECK_ARG(ld_q % 8 == 0 && ld_kv % 8 == 0 && ld_out % 8 == 0, "spb_attention_decode: leading dims must be multiples of 8");
+    SPB_CHECK_ARG(pos_dev != nullptr || !append_kv || (q_pos >= 0 && q_pos < n_keys),
+                  "spb_attention_decode: append_kv needs 0 <= q_pos < n_keys, got q_pos %d, n_keys %d", q_pos, n_keys);
     const size_t smem = (size_t)H * n_keys * sizeof(float);
+    static int smem_max = 0;
+    if (smem_max == 0) {
+        int dev = 0;
+        SPB_CHECK_CUDA(cudaGetDevice(&dev));
+        SPB_CHECK_CUDA(cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+    }
+    SPB_CHECK_ARG(smem <= (size_t)smem_max, "spb_attention_decode: %d heads x %d keys need %zu bytes of shared memory, the device has %d per block",
+                  H, n_keys, smem, smem_max);
     static size_t configured = 48 * 1024;
     if (smem > configured) {
         SPB_CHECK_CUDA(cudaFuncSetAttribute(attn_decode_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));

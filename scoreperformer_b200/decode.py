@@ -21,6 +21,9 @@ from torch import Tensor
 from . import fused, kernels as K
 
 BF16, F32 = torch.bfloat16, torch.float32
+# largest bf16 [B, T, (2 depth + 1) 512] table of AdaLN terms render_decoder prepares ahead of its loop; a larger rendering has the
+# stack kernel evaluate them step by step
+ADALN_TERMS_MAX_BYTES = 8 << 30
 
 
 class _StackWeights:
@@ -209,21 +212,20 @@ def render_decoder(dec, perf: Tensor, masked_perf: Tensor, score_hidden: Tensor,
         assert init.shape == (B, start, 128)
         kv[:, :start] = init
     out = perf.clone()
-    feed = out if teacher is None else teacher
-    cat_buf = torch.empty((B, 2 * dec.dim), dtype=BF16, device=dev)
-    cat2 = torch.empty((B, 2 * dec.dim), dtype=BF16, device=dev)
+    feed = (out if teacher is None else teacher).contiguous()
 
     # The position lives on the device: every index below is a device gather / scatter, so ONE captured step replays for
     # all T-1 notes (`use_graph`), instead of ~50 host launches per note.
     pos_t = torch.full((1,), start, dtype=torch.int64, device=dev)           # i
     field_idx = torch.tensor(list(fields), dtype=torch.int64, device=dev)
     neg_inf = -float("inf")
-
-    # the whole decoder stack of a note-step is ONE persistent kernel when the stack has the recipe's shape (csrc/decode_stack.cu);
-    # SPB_DECODE=legacy keeps the launch-per-operator path (also the fallback for other shapes)
-    plan = None
     style_f = style.float().contiguous()
-    if K.decode_stack_ok(sw.depth, sw.D, sw.H, sw.layers[0]["w2"].shape[1], sw.ada, style_f.shape[-1], T):
+
+    # SPB_DECODE=legacy runs the launch-per-operator stack and samples on the host side: the reference of the parity tests
+    legacy = K._os.environ.get("SPB_DECODE", "fused") != "fused"
+    # the whole decoder stack of a note-step is ONE persistent kernel when the stack has the recipe's shape (csrc/decode_stack.cu)
+    plan = None
+    if not legacy and K.decode_stack_ok(sw.depth, sw.D, sw.H, sw.layers[0]["w2"].shape[1], sw.ada, style_f.shape[-1], T):
         plan = K.DecodeStackPlan(sw.layers, sw.w_ada, sw.b_ada, kv_caches, B, style_f.shape[-1])
 
     filtered = top_p is not None or top_a is not None
@@ -234,128 +236,110 @@ def render_decoder(dec, perf: Tensor, masked_perf: Tensor, score_hidden: Tensor,
     else:
         ks = [int(k) for k in top_k]
         assert len(ks) == len(fields), "top_k: one k per rendered field"
-    fused_sampling = (generator is None and emb == 128 and len(fields) <= 8 and all(sizes[f] <= 256 for f in fields)
-                      and all(1 <= k <= 32 for k in ks) and K._os.environ.get("SPB_DECODE", "fused") == "fused")
+    fused_sampling = (not legacy and generator is None and emb == 128 and len(fields) <= 8 and all(sizes[f] <= 256 for f in fields)
+                      and all(1 <= k <= 32 for k in ks))
     seed = K.seed_from_torch() if filtered or any(k > 1 for k in ks) else 0
     # the filters and bans of the sampling launch (all None: the plain top-k call)
     filt_kw = dict(top_p=None if top_p is None else [float(top_p)] * len(fields),
                    top_a=None if top_a is None else [(float(top_a[0]), float(top_a[1]))] * len(fields),
                    banned=bans if any(bans) else None)
     ban_idx = {f: torch.tensor(ids, dtype=torch.int64, device=dev) for f, ids in zip(fields, bans) if ids}
+    # with the stack kernel and the sampling kernel both in the step, the sampling kernel's last CTA ends the step: position += 1,
+    # grid-barrier word of the stack kernel back to zero
+    sampler_ends_step = plan is not None and fused_sampling
 
     # Everything of a note-step that does not depend on the tokens sampled so far is evaluated for ALL positions before the loop,
     # in large launches: the masked tuple of note i+1 through the embedding and its half of project_multiemb (+ bias), and the
     # context half of project_emb (+ bias).  A step then adds its own half (the previous, complete tuple) as a GEMM with a residual.
-    lean = plan is not None
-    if lean:
-        Dm = dec.dim
-        wm_r, wc_l, wc_r = wm16[:, Dm:], wc16[:, :Dm], wc16[:, Dm:]
-        # project_emb of the tuple embedding and the left half of project_multiemb are two linear maps in a row: composed once per
-        # rendering in fp32 (W = Wm_left Wp, its bias joins the prepared term), so a step needs one GEMM for both
-        wm_full = te_mod.project_multiemb.weight.detach().float()
-        w_comp16 = K.cast_bf16((wm_full[:, :Dm] @ te_mod.project_emb.weight.detach().float()).contiguous())        # [D, F * 128]
-        b_comp = (wm_full[:, :Dm] @ bp.float()).contiguous()                                                          # [D]
-        P2 = torch.empty((B, T, Dm), dtype=F32, device=dev)
-        C2 = torch.empty((B, T, Dm), dtype=F32, device=dev)
-        cb = max(1, min(B, 32768 // max(T, 1)))
-        for b0 in range(0, B, cb):
-            b1 = min(B, b0 + cb)
-            x2, _, _ = K.embed_ln_fwd(masked_perf[b0:b1].reshape(-1, F).contiguous(), table, sizes, ln_w, ln_b)
-            x2p = K.gemm(x2, wp16, bias=bp, out_dtype=BF16)
-            K.gemm(x2p, wm_r, bias=bm + b_comp, out=P2[b0:b1].view(-1, Dm))
-            K.gemm(ctx16[b0:b1].reshape(-1, ctx16.shape[-1]), wc_r, bias=bc, out=C2[b0:b1].view(-1, Dm))
-            del x2, x2p
-        # ... and the AdaLN terms of every position (one GEMM instead of a tile phase per step), memory permitting
-        gb_all = None
-        if B * T * plan.gb.shape[1] * 2 <= int(K._os.environ.get("SPB_DECODE_GB_ALL_BYTES", str(8 << 30))):
-            gb_all = plan.prepare_adaln(style_f)
-        feed_c = feed.contiguous()
-        tok_buf = torch.empty((B, F), dtype=feed_c.dtype, device=dev)
-        p2_buf = torch.empty((B, Dm), dtype=F32, device=dev)
-        c2_buf = torch.empty((B, Dm), dtype=F32, device=dev)
+    Dm = dec.dim
+    wm_r, wc_l, wc_r = wm16[:, Dm:], wc16[:, :Dm], wc16[:, Dm:]
+    # project_emb of the tuple embedding and the left half of project_multiemb are two linear maps in a row: composed once per
+    # rendering in fp32 (W = Wm_left Wp, its bias joins the prepared term), so a step needs one GEMM for both
+    wm_full = te_mod.project_multiemb.weight.detach().float()
+    w_comp16 = K.cast_bf16((wm_full[:, :Dm] @ te_mod.project_emb.weight.detach().float()).contiguous())        # [D, F * 128]
+    b_comp = (wm_full[:, :Dm] @ bp.float()).contiguous()                                                          # [D]
+    P2 = torch.empty((B, T, Dm), dtype=F32, device=dev)
+    C2 = torch.empty((B, T, Dm), dtype=F32, device=dev)
+    cb = max(1, min(B, 32768 // max(T, 1)))
+    for b0 in range(0, B, cb):
+        b1 = min(B, b0 + cb)
+        x2, _, _ = K.embed_ln_fwd(masked_perf[b0:b1].reshape(-1, F).contiguous(), table, sizes, ln_w, ln_b)
+        x2p = K.gemm(x2, wp16, bias=bp, out_dtype=BF16)
+        K.gemm(x2p, wm_r, bias=bm + b_comp, out=P2[b0:b1].view(-1, Dm))
+        K.gemm(ctx16[b0:b1].reshape(-1, ctx16.shape[-1]), wc_r, bias=bc, out=C2[b0:b1].view(-1, Dm))
+        del x2, x2p
+    # ... and the AdaLN terms of every position for the stack kernel (one GEMM instead of a tile phase per step), memory permitting
+    gb_all = None
+    if plan is not None and B * T * plan.gb.shape[1] * 2 <= ADALN_TERMS_MAX_BYTES:
+        gb_all = plan.prepare_adaln(style_f)
+    # one launch per step reads what the step needs at the device-side position: tuple i, and the prepared terms / style of note i+1
+    tok_buf = torch.empty((B, F), dtype=feed.dtype, device=dev)
+    p2_buf = torch.empty((B, Dm), dtype=F32, device=dev)
+    c2_buf = torch.empty((B, Dm), dtype=F32, device=dev)
+    gather_src, gather_dst = [feed, P2, C2], [tok_buf, p2_buf, c2_buf]
+    st_buf = None
+    if gb_all is None:
         st_buf = torch.empty((B, style_f.shape[-1]), dtype=F32, device=dev)
-        ln_buf = torch.empty((B, Dm), dtype=BF16, device=dev)
-        # the rest of the front (te = x1 W^T + p2, emb_norm, project_emb's left half + c2) runs inside the stack kernel when the
-        # tuple embedding has the recipe's width; x1 is then a static buffer the embedding kernel fills
-        front_in_kernel = gb_all is not None and len(sizes) * 128 == 1536 and Dm == 256 \
-            and K._os.environ.get("SPB_DECODE_FRONT_IN_KERNEL", "1") == "1"
-        if front_in_kernel:
-            x1_buf = torch.empty((B, 1536), dtype=BF16, device=dev)
-            plan.set_front(x1_buf, w_comp16, p2_buf, en_w.float().contiguous(), en_b.float().contiguous(), wc_l.t().contiguous(), c2_buf)
+        gather_src.append(style_f)
+        gather_dst.append(st_buf)
+    gather_shift = [0] + [1] * (len(gather_src) - 1)
+    ln_buf = torch.empty((B, Dm), dtype=BF16, device=dev)
+    # the rest of the front (te = x1 W^T + p2, emb_norm, project_emb's left half + c2) runs inside the stack kernel when the
+    # tuple embedding has the recipe's width; x1 is then a static buffer the embedding kernel fills
+    front_in_kernel = gb_all is not None and len(sizes) * 128 == 1536 and Dm == 256
+    if front_in_kernel:
+        x1_buf = torch.empty((B, 1536), dtype=BF16, device=dev)
+        plan.set_front(x1_buf, w_comp16, p2_buf, en_w.float().contiguous(), en_b.float().contiguous(), wc_l.t().contiguous(), c2_buf)
 
-    def step_lean():
-        # one launch reads what this step needs at the device-side position: tuple i, and the prepared terms / style of note i+1
-        if gb_all is None:
-            K.gather_at_pos([feed_c, P2, C2, style_f], [tok_buf, p2_buf, c2_buf, st_buf], [0, 1, 1, 1], pos_t)
-        else:
-            K.gather_at_pos([feed_c, P2, C2], [tok_buf, p2_buf, c2_buf], [0, 1, 1], pos_t)
+    def sample_on_host(e):
+        # heads of the rendered fields, PAD / MASK and per-field bans, logit filter and draw in torch; out[:, i+1, fields] = toks
+        toks = []
+        for f, k in zip(fields, ks):
+            lg = K.gemm(e[:, f * emb:(f + 1) * emb], table16[offs[f]:offs[f] + sizes[f]], out_dtype=F32)
+            lg[:, :2] = neg_inf                                                 # PAD / MASK are never emitted
+            if f in ban_idx:
+                lg.index_fill_(1, ban_idx[f], neg_inf)
+            if filtered:
+                lg = sampling.top_p(lg, float(top_p)) if top_p is not None else _top_a_rows(lg, *top_a)
+                tok = torch.multinomial(torch.softmax(lg / temperature, dim=-1), 1, generator=generator).squeeze(1)
+            elif k == 1:
+                tok = lg.argmax(dim=-1)
+            else:
+                val, ind = torch.topk(lg, k)
+                probs = torch.softmax(val / temperature, dim=-1)
+                tok = ind.gather(1, torch.multinomial(probs, 1, generator=generator)).squeeze(1)
+            toks.append(tok)
+        dst = (pos_t + 1) * F + field_idx                                       # [n_fields] flat column indices
+        out.view(B, T * F).index_copy_(1, dst, torch.stack(toks, dim=1))
+
+    def step():
+        # decoder position i: full tuple of note i, masked tuple / context / style of note i+1 (wrappers.py:409-431)
+        K.gather_at_pos(gather_src, gather_dst, gather_shift, pos_t)
         if front_in_kernel:
             K.embed_ln_fwd(tok_buf, table, sizes, ln_w, ln_b, out=x1_buf)
-            plan.step(None, None, km, pos_t, gb_all=gb_all, use_front=True, barrier_is_zero=True)
+            x = None
         else:
             x1, _, _ = K.embed_ln_fwd(tok_buf, table, sizes, ln_w, ln_b)
             te = K.gemm(x1, w_comp16, residual=p2_buf, out_dtype=F32)
             K.layer_norm_fwd(te, en_w, en_b, out=ln_buf, need_stats=False)
             x = K.gemm(ln_buf, wc_l, residual=c2_buf, out_dtype=F32)
-            plan.step(x, st_buf if gb_all is None else None, km, pos_t, gb_all=gb_all)
-        # tied head for the masked fields only (wrappers.py:364-380); the stack kernel leaves a bf16 copy of its output
-        e_raw = K.gemm(plan.out16, whead16, trans_b=True, out_dtype=BF16)
-        e, _, _ = K.layer_norm_fwd(e_raw, hn_w, hn_b, out_dtype=BF16, need_stats=False)
-        if front_in_kernel:
-            # the sampling kernel's last CTA ends the step: position += 1, grid-barrier word of the stack kernel back to zero
-            K.sample_fields(e, table16, fields, [offs[f] for f in fields], [sizes[f] for f in fields], ks, out, pos_t,
-                            temperature=temperature, seed=seed, advance=plan.advance, **filt_kw)
-        else:
-            K.sample_fields(e, table16, fields, [offs[f] for f in fields], [sizes[f] for f in fields], ks, out, pos_t,
-                            temperature=temperature, seed=seed, **filt_kw)
-            pos_t.add_(1)
-
-    def step():
-        if lean and fused_sampling and (feed_c is out or teacher is not None):
-            return step_lean()
-        nxt = pos_t + 1
-        # decoder position i: full tuple of note i, masked tuple / context / style of note i+1 (wrappers.py:409-431)
-        x1, _, _ = K.embed_ln_fwd(feed.index_select(1, pos_t).reshape(B, F).contiguous(), table, sizes, ln_w, ln_b)
-        x2, _, _ = K.embed_ln_fwd(masked_perf.index_select(1, nxt).reshape(B, F).contiguous(), table, sizes, ln_w, ln_b)
-        K.gemm(x1, wp16, bias=bp, out=cat_buf[:, :dec.dim])
-        K.gemm(x2, wp16, bias=bp, out=cat_buf[:, dec.dim:])
-        te = K.gemm(cat_buf, wm16, bias=bm, out_dtype=F32)
-        K.layer_norm_fwd(te, en_w, en_b, out=cat2[:, :dec.dim], need_stats=False)
-        cat2[:, dec.dim:].copy_(ctx16.index_select(1, nxt).reshape(B, -1))
-        x = K.gemm(cat2, wc16, bias=bc, out_dtype=F32)
         if plan is not None:
-            hid = plan.step(x, style_f.index_select(1, nxt).reshape(B, -1), km, pos_t)
+            # the stack kernel leaves a bf16 copy of its output, the head projection's operand
+            plan.step(x, st_buf, km, pos_t, gb_all=gb_all, use_front=front_in_kernel, barrier_is_zero=sampler_ends_step)
+            hid16 = plan.out16
         else:
-            hid = _stack_step(sw, x, style.index_select(1, nxt).reshape(B, -1), kv_caches, km, 0, pos_dev=pos_t)
+            hid16 = K.cast_bf16(_stack_step(sw, x, st_buf, kv_caches, km, 0, pos_dev=pos_t))
         # tied head for the masked fields only (wrappers.py:364-380)
-        e_raw = K.gemm(K.cast_bf16(hid), whead16, trans_b=True, out_dtype=BF16)
+        e_raw = K.gemm(hid16, whead16, trans_b=True, out_dtype=BF16)
         e, _, _ = K.layer_norm_fwd(e_raw, hn_w, hn_b, out_dtype=BF16, need_stats=False)
         if fused_sampling:
             # heads of the rendered fields, PAD / MASK and per-field bans, logit filter, draw and token write: one launch
             K.sample_fields(e, table16, fields, [offs[f] for f in fields], [sizes[f] for f in fields], ks, out, pos_t,
-                            temperature=temperature, seed=seed, **filt_kw)
+                            temperature=temperature, seed=seed, advance=plan.advance if sampler_ends_step else None, **filt_kw)
         else:
-            toks = []
-            for f, k in zip(fields, ks):
-                lg = K.gemm(e[:, f * emb:(f + 1) * emb], table16[offs[f]:offs[f] + sizes[f]], out_dtype=F32)
-                lg[:, :2] = neg_inf                                             # PAD / MASK are never emitted
-                if f in ban_idx:
-                    lg.index_fill_(1, ban_idx[f], neg_inf)
-                if filtered:
-                    lg = sampling.top_p(lg, float(top_p)) if top_p is not None else _top_a_rows(lg, *top_a)
-                    tok = torch.multinomial(torch.softmax(lg / temperature, dim=-1), 1, generator=generator).squeeze(1)
-                elif k == 1:
-                    tok = lg.argmax(dim=-1)
-                else:
-                    val, ind = torch.topk(lg, k)
-                    probs = torch.softmax(val / temperature, dim=-1)
-                    tok = ind.gather(1, torch.multinomial(probs, 1, generator=generator)).squeeze(1)
-                toks.append(tok)
-            # out[:, i+1, fields] = toks
-            out_rows = out.view(B, T * F)
-            dst = nxt * F + field_idx                                           # [n_fields] flat column indices
-            out_rows.index_copy_(1, dst, torch.stack(toks, dim=1))
-        pos_t.add_(1)
+            sample_on_host(e)
+        if not sampler_ends_step:
+            pos_t.add_(1)
 
     n_steps = T - 1 - start
     # host-side filters sort and mask with data-dependent shapes: that step runs eagerly

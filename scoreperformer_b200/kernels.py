@@ -284,7 +284,7 @@ def sample_fields(e: Tensor, table16: Tensor, fields: Sequence[int], offsets: Se
 
 def decode_stack_ok(depth: int, dim: int, heads: int, hidden: int, ada: bool, style_dim: int, cap: int) -> bool:
     return (ada and dim == 256 and heads == 4 and hidden == 1024 and 1 <= depth <= 8 and style_dim % 16 == 0 and 16 <= style_dim <= 256
-            and cap <= 2048 and _os.environ.get("SPB_DECODE", "fused") == "fused")
+            and cap <= 2048)
 
 
 # ----------------------------------------------------------------------------- collator (device side)

@@ -95,6 +95,14 @@ int spb_decode_stack_step(const float* x_in, const float* style, int S, const vo
  * its device-side position. */
 int spb_gather_at_pos(const void* const* srcs, void* const* dsts, const int* row_bytes, const int* shifts, int n, const long long* pos_dev,
                       int B, int T, spb_stream_t stream);
+/* Start of a streaming call of a render session that keeps staged weights across calls, one launch: hashes the bit patterns of
+ * n_tensors tensors (table = DEVICE int64 [n_tensors, 3]: device address, number of 32-bit words, index of its first word) into
+ *     fingerprint = sum over words i of splitmix64((i << 32) | word_i)  mod 2^64
+ * (order-independent, so CTAs combine with integer atomics), then state[3] = (fingerprint != state[0]) and state[0] = fingerprint.
+ * state: device uint64 [4]; state[1] and state[2] must be zero on entry and are zero again on return.  Also clears advance[0..1] (the
+ * counter of spb_sample_fields and the grid-barrier word of spb_decode_stack_step) and sets *pos_dev = start. */
+int spb_session_begin(const long long* table, int n_tensors, unsigned long long* state, unsigned* advance, long long* pos_dev,
+                      long long start, spb_stream_t stream);
 
 /* Tied heads of the rendered fields + sampling in one launch (modules/sampling.py:12-59, wrappers.py:358-397): per listed field
  * (host int arrays: field index, first table row, vocabulary <= 256, top-k <= 32; k = 1 is greedy) logits = e_f . table_f^T stay in

@@ -1230,3 +1230,94 @@ extern "C" int spb_sample_fields_filtered(const void* e, int ld_e, const void* t
     return launch_sample_fields("spb_sample_fields_filtered", e, ld_e, table, fields, offsets, vocab, topk, n_fields, n_banned, temperature,
                                 seed, pos_dev, tokens, B, T, F, advance, top_p, top_a_pow, top_a_ratio, ban_bits, stream);
 }
+
+// ============================================================================================================================
+// Start of a streaming call of a render session (decode.py `_RenderSession`): the session keeps bf16 copies of the decoder's
+// weights and a stack plan between calls, so before it enqueues the note-steps it has to know whether the weights moved under it.
+// torch's version counters do not tell (the flat AdamW kernel writes parameters through raw pointers), so this launch hashes the
+// bit patterns of every parameter and buffer of the decoder into a 64-bit fingerprint:
+//     fingerprint = sum over words i of splitmix64((i << 32) | word_i)   (mod 2^64)
+// where i numbers the 32-bit words of all listed tensors in table order.  The index mixing makes a moved value count; the sum is
+// order-independent, so CTAs hash any slice they like and meet in one integer atomic.  The last CTA compares the fingerprint with
+// the stored one, writes the stale flag the host reads, and stores the new fingerprint.  The same launch also zeroes the stack
+// plan's `advance` words (sample_fields' CTA counter and the stack kernel's grid-barrier word: a plan that outlives a call must not
+// rely on the sampler of an earlier call having cleared them) and writes the call's start position.
+namespace {
+
+constexpr int SB_THREADS = 256;
+
+struct SessionBeginParams {
+    const long long* table;       // [n, 3]: device address, number of 32-bit words, index of the first word
+    int n;
+    unsigned long long* state;    // [4]: stored fingerprint, running sum, finished CTAs (both zero between launches), stale flag
+    unsigned* advance;            // [2]
+    long long* pos_dev;
+    long long start;
+};
+
+__device__ __forceinline__ unsigned long long fingerprint_term(unsigned long long index, unsigned word) {
+    unsigned long long z = ((index << 32) | word) + 0x9E3779B97F4A7C15ull;
+    z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+    z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
+    return z ^ (z >> 31);
+}
+
+__global__ void __launch_bounds__(SB_THREADS) session_begin_kernel(SessionBeginParams p) {
+    if (blockIdx.x == 0 && threadIdx.x == 0) {
+        p.advance[0] = 0u;
+        p.advance[1] = 0u;
+        *p.pos_dev = p.start;
+    }
+    const long long tid = (long long)blockIdx.x * SB_THREADS + threadIdx.x, nth = (long long)gridDim.x * SB_THREADS;
+    unsigned long long acc = 0;
+    for (int t = 0; t < p.n; ++t) {
+        const unsigned* w = reinterpret_cast<const unsigned*>(p.table[3 * t]);
+        const long long n = p.table[3 * t + 1];
+        const unsigned long long first = (unsigned long long)p.table[3 * t + 2];
+        long long done = 0;
+        if ((reinterpret_cast<uintptr_t>(w) & 15) == 0) {         // 16-byte loads over the aligned body
+            const uint4* w4 = reinterpret_cast<const uint4*>(w);
+            const long long n4 = n >> 2;
+            for (long long i = tid; i < n4; i += nth) {
+                const uint4 v = __ldg(w4 + i);
+                const unsigned long long g = first + 4ull * (unsigned long long)i;
+                acc += fingerprint_term(g, v.x) + fingerprint_term(g + 1, v.y) + fingerprint_term(g + 2, v.z) + fingerprint_term(g + 3, v.w);
+            }
+            done = n4 << 2;
+        }
+        for (long long i = done + tid; i < n; i += nth) acc += fingerprint_term(first + (unsigned long long)i, __ldg(w + i));
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+    __shared__ unsigned long long s_part[SB_THREADS / 32];
+    if ((threadIdx.x & 31) == 0) s_part[threadIdx.x >> 5] = acc;
+    __syncthreads();
+    if (threadIdx.x != 0) return;
+    unsigned long long sum = 0;
+#pragma unroll
+    for (int i = 0; i < SB_THREADS / 32; ++i) sum += s_part[i];
+    atomicAdd(p.state + 1, sum);
+    __threadfence();
+    if (atomicAdd(p.state + 2, 1ull) != gridDim.x - 1) return;
+    // the last CTA: every other CTA added its part before it counted itself in
+    __threadfence();
+    const unsigned long long fp = atomicExch(p.state + 1, 0ull);
+    p.state[3] = fp != p.state[0] ? 1ull : 0ull;
+    p.state[0] = fp;
+    p.state[2] = 0ull;
+}
+
+}  // namespace
+
+// table: DEVICE int64 [n_tensors, 3] (address, number of 32-bit words, index of the first word); state: device uint64 [4] (stored
+// fingerprint, two words that must be zero between launches, stale flag written here); advance: the stack plan's uint32 [2];
+// pos_dev: device int64 set to `start`.
+extern "C" int spb_session_begin(const long long* table, int n_tensors, unsigned long long* state, unsigned* advance, long long* pos_dev,
+                                 long long start, cudaStream_t stream) {
+    SPB_CHECK_ARG(table && state && advance && pos_dev && n_tensors >= 0 && start >= 0, "spb_session_begin: bad arguments");
+    SessionBeginParams p;
+    p.table = table; p.n = n_tensors; p.state = state; p.advance = advance; p.pos_dev = pos_dev; p.start = start;
+    session_begin_kernel<<<4 * spb_num_sms(), SB_THREADS, 0, stream>>>(p);
+    SPB_CHECK_LAUNCH();
+    return SPB_OK;
+}

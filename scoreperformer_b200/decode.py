@@ -13,6 +13,7 @@ Two entry points over the same kernels:
 from __future__ import annotations
 
 import math
+import weakref
 from typing import Callable, Dict, List, Optional, Sequence, Tuple, Union
 
 import torch
@@ -62,6 +63,45 @@ class _StackWeights:
             gb = gb_all[:, i * 2 * self.D:(i + 1) * 2 * self.D]
             return K.layer_norm_fwd(x, None, None, gb, out_dtype=out_dtype, need_stats=False)[0]
         return K.layer_norm_fwd(x, self.norm_w[i], self.norm_b[i], out_dtype=out_dtype, need_stats=False)[0]
+
+
+class _DecoderWeights:
+    """What a rendering stages from the performance decoder's parameters before its note loop: the stack's bf16 weights, the
+    computed token table (value MLPs) and its bf16 copy, bf16 copies of the front / head projections.  Biases and norm weights are
+    views of the parameters."""
+
+    def __init__(self, dec):
+        te_mod, head = dec.token_emb, dec.lm_head
+        self.sw = _StackWeights(dec.transformer)
+        self.table = te_mod.table().detach().contiguous()
+        self.table16 = K.cast_bf16(self.table)
+        self.ln_w, self.ln_b = te_mod.norm.weight.detach(), te_mod.norm.bias.detach()
+        self.wp16 = K.cast_bf16(te_mod.project_emb.weight.detach().contiguous())
+        self.bp = te_mod.project_emb.bias.detach()
+        self.wm16 = K.cast_bf16(te_mod.project_multiemb.weight.detach().contiguous())
+        self.bm = te_mod.project_multiemb.bias.detach()
+        self.en_w, self.en_b = dec.emb_norm.weight.detach(), dec.emb_norm.bias.detach()
+        self.wc16 = K.cast_bf16(dec.project_emb.weight.detach().contiguous())
+        self.bc = dec.project_emb.bias.detach()
+        self.whead16 = K.cast_bf16(head.proj_weight_kn().detach().contiguous())
+        self.hn_w, self.hn_b = head.norm.weight.detach(), head.norm.bias.detach()
+        self.emb = head.split_dims[0]
+        self.offs = [0]
+        for v in te_mod.field_sizes[:-1]:
+            self.offs.append(self.offs[-1] + v)
+        Dm = dec.dim
+        self.wm_r, self.wc_l, self.wc_r = self.wm16[:, Dm:], self.wc16[:, :Dm], self.wc16[:, Dm:]
+        self._te_mod, self._Dm = te_mod, Dm
+
+    def compose_front(self) -> Tuple[Tensor, Tensor]:
+        """project_emb of the tuple embedding and the left half of project_multiemb are two linear maps in a row: composed in fp32
+        (W = Wm_left Wp, its bias joins the prepared term), so a note-step needs one GEMM for both.  Returns (W bf16 [D, F * 128],
+        bias fp32 [D])."""
+        te_mod, Dm = self._te_mod, self._Dm
+        wm_full = te_mod.project_multiemb.weight.detach().float()
+        w_comp16 = K.cast_bf16((wm_full[:, :Dm] @ te_mod.project_emb.weight.detach().float()).contiguous())        # [D, F * 128]
+        b_comp = (wm_full[:, :Dm] @ self.bp.float()).contiguous()                                                     # [D]
+        return w_comp16, b_comp
 
 
 def _stack_step(sw: _StackWeights, x_last: Tensor, style_last: Optional[Tensor], kv_caches: Sequence[Tensor], key_mask: Optional[Tensor],
@@ -182,28 +222,14 @@ def render_decoder(dec, perf: Tensor, masked_perf: Tensor, score_hidden: Tensor,
     are rendered).  `return_kv` also returns the per-layer caches [B, T, 128] (rows < T-1 valid).
     """
     from .modules import sampling
-    te_mod, head = dec.token_emb, dec.lm_head
-    sizes = te_mod.field_sizes
+    sizes = dec.token_emb.field_sizes
     bans = _check_filters(top_k, top_p, top_a, banned_tokens, fields, sizes)
     B, T, F = perf.shape
     dev = perf.device
-    sw = _StackWeights(dec.transformer)
-    table = te_mod.table().detach().contiguous()
-    table16 = K.cast_bf16(table)
-    ln_w, ln_b = te_mod.norm.weight.detach(), te_mod.norm.bias.detach()
-    wp16 = K.cast_bf16(te_mod.project_emb.weight.detach().contiguous())
-    bp = te_mod.project_emb.bias.detach()
-    wm16 = K.cast_bf16(te_mod.project_multiemb.weight.detach().contiguous())
-    bm = te_mod.project_multiemb.bias.detach()
-    en_w, en_b = dec.emb_norm.weight.detach(), dec.emb_norm.bias.detach()
-    wc16 = K.cast_bf16(dec.project_emb.weight.detach().contiguous())
-    bc = dec.project_emb.bias.detach()
-    whead16 = K.cast_bf16(head.proj_weight_kn().detach().contiguous())
-    hn_w, hn_b = head.norm.weight.detach(), head.norm.bias.detach()
-    emb = head.split_dims[0]
-    offs = [0]
-    for v in sizes[:-1]:
-        offs.append(offs[-1] + v)
+    st = _DecoderWeights(dec)
+    sw, table, table16, ln_w, ln_b, wp16, bp, bm = st.sw, st.table, st.table16, st.ln_w, st.ln_b, st.wp16, st.bp, st.bm
+    en_w, en_b, wc16, bc, whead16, hn_w, hn_b = st.en_w, st.en_b, st.wc16, st.bc, st.whead16, st.hn_w, st.hn_b
+    emb, offs = st.emb, st.offs
     ctx16 = K.cast_bf16(score_hidden.float().contiguous().view(B * T, -1)).view(B, T, -1)
     km = None if mask is None else mask.contiguous()
     kv_caches = [torch.zeros((B, T, 128), dtype=BF16, device=dev) for _ in range(sw.depth)]
@@ -252,12 +278,8 @@ def render_decoder(dec, perf: Tensor, masked_perf: Tensor, score_hidden: Tensor,
     # in large launches: the masked tuple of note i+1 through the embedding and its half of project_multiemb (+ bias), and the
     # context half of project_emb (+ bias).  A step then adds its own half (the previous, complete tuple) as a GEMM with a residual.
     Dm = dec.dim
-    wm_r, wc_l, wc_r = wm16[:, Dm:], wc16[:, :Dm], wc16[:, Dm:]
-    # project_emb of the tuple embedding and the left half of project_multiemb are two linear maps in a row: composed once per
-    # rendering in fp32 (W = Wm_left Wp, its bias joins the prepared term), so a step needs one GEMM for both
-    wm_full = te_mod.project_multiemb.weight.detach().float()
-    w_comp16 = K.cast_bf16((wm_full[:, :Dm] @ te_mod.project_emb.weight.detach().float()).contiguous())        # [D, F * 128]
-    b_comp = (wm_full[:, :Dm] @ bp.float()).contiguous()                                                          # [D]
+    wm_r, wc_l, wc_r = st.wm_r, st.wc_l, st.wc_r
+    w_comp16, b_comp = st.compose_front()
     P2 = torch.empty((B, T, Dm), dtype=F32, device=dev)
     C2 = torch.empty((B, T, Dm), dtype=F32, device=dev)
     cb = max(1, min(B, 32768 // max(T, 1)))
@@ -439,9 +461,16 @@ def unmask_mixlm(wrapper, tokens: Tensor, tokens_masked: Tensor, temperature: fl
     expressible = (ks is not None and not filter_key_ids and contiguous_tail and uniform and context is not None and style is not None
                    and len(set(ks)) == 1 and set(kwargs) <= {"context", "style_embeddings"})
     fast = expressible and caches is None and not return_caches and int(notes[0]) == 1
-    kv_init = _streamable(dec, caches, int(notes[0]) - 1, context, style, T) if expressible and not fast else None
+    start = int(notes[0]) - 1 if notes.numel() else 0
+    att = _stream_prefix(dec, caches, start, context, style, T) if expressible and not fast else None
+    session = _session_for(dec, out, fields, ks[0], style) if att is not None else None
+    kv_init = None if att is None or session is not None else _streamable(dec, caches, start, context, style, T)
     if fast:
         res = render_decoder(dec, out, tokens_masked, context, style, mask=mask, fields=fields, temperature=temperature, top_k=ks[0])
+    elif session is not None:
+        # the streaming call of inference/generators.py on the decoder's render session: staged weights, stack plan and buffers are
+        # kept between calls, the keys / values of a prefix the session handed out are continued in place
+        res, caches = session.render(dec, out, tokens_masked, context, style, mask, fields, temperature, ks[0], start, caches)
     elif kv_init is not None:
         # the streaming call of inference/generators.py: a few new notes behind a prefix whose keys / values the caller holds.  Same
         # device-resident note-step as a whole-window rendering (persistent stack kernel, fused heads + sampling), started at the
@@ -457,10 +486,11 @@ def unmask_mixlm(wrapper, tokens: Tensor, tokens_masked: Tensor, temperature: fl
     return (res, caches) if return_caches else res
 
 
-def _streamable(dec, caches, start: int, context: Tensor, style: Tensor, T: int):
-    """Per-layer [B, start, 128] keys | values if the request can continue on the device-resident note-step: nothing cached and the
-    first note is the one to render, or caches whose length is exactly the known prefix (the check inference/generators.py:222-226
-    makes as well).  None sends the request to the general stepper.  SPB_STREAM=legacy switches this path off."""
+def _stream_prefix(dec, caches, start: int, context: Tensor, style: Tensor, T: int):
+    """The per-layer AttentionIntermediates of the prefix ([] when nothing is cached) if the request can continue on the
+    device-resident note-step: nothing cached and the first note is the one to render, or caches whose length is exactly the known
+    prefix (the check inference/generators.py:222-226 makes as well).  None sends the request to the general stepper.
+    SPB_STREAM=legacy switches this path off."""
     if K._os.environ.get("SPB_STREAM", "fused") != "fused" or context.shape[1] != T or style.shape[1] != T or start < 0:
         return None
     if caches is None:
@@ -470,22 +500,209 @@ def _streamable(dec, caches, start: int, context: Tensor, style: Tensor, T: int)
         return None
     if any(a.keys is None or a.values is None or a.keys.shape[-2] != start for a in att):
         return None
-    return [torch.cat([a.keys, a.values], dim=-1).to(BF16).contiguous() for a in att]
+    return att
 
 
-def _kv_only_caches(dec, kvs: Sequence[Tensor], length: int):
+def _streamable(dec, caches, start: int, context: Tensor, style: Tensor, T: int):
+    """Per-layer [B, start, 128] keys | values of `_stream_prefix`, or None."""
+    att = _stream_prefix(dec, caches, start, context, style, T)
+    return None if att is None else [torch.cat([a.keys, a.values], dim=-1).to(BF16).contiguous() for a in att]
+
+
+def _kv_only_caches(dec, kvs: Sequence[Tensor], length: int, zeros: Optional[Tensor] = None):
     """Caches in the reference's layout (TupleTransformerCaches / TransformerIntermediates / AttentionIntermediates, every tensor
     [B, length, .]) after a device-resident rendering.  Keys and values are views of the working buffers.  `token_emb` and `hiddens`
-    are ZERO placeholders of the right shapes: the cached step of this implementation needs the keys and values of the prefix and
-    the last position only (the reference recomputes emb_norm / project_emb over the whole prefix from `token_emb` at every step,
-    transformer.py:171-185, and carries the per-layer hiddens without reading them)."""
+    are ZERO placeholders of the right shapes (views of `zeros` [B, >= length, dim] when given): the cached step of this
+    implementation needs the keys and values of the prefix and the last position only (the reference recomputes emb_norm /
+    project_emb over the whole prefix from `token_emb` at every step, transformer.py:171-185, and carries the per-layer hiddens
+    without reading them)."""
     from .models.scoreperformer.transformer import TupleTransformerCaches
     from .modules.transformer.attend import AttentionIntermediates
     from .modules.transformer.transformer import TransformerIntermediates
     B = kvs[0].shape[0]
-    z = torch.zeros((B, length, dec.dim), dtype=F32, device=kvs[0].device)
+    z = torch.zeros((B, length, dec.dim), dtype=F32, device=kvs[0].device) if zeros is None else zeros[:, :length]
     att = [AttentionIntermediates(keys=kv[:, :length, :64], values=kv[:, :length, 64:]) for kv in kvs]
     return TupleTransformerCaches(token_emb=z, transformer=TransformerIntermediates(hiddens=[z] * (len(kvs) + 1), attention=att))
+
+
+# ----------------------------------------------------------------------------- render sessions (streaming calls)
+# A real-time rendering calls `unmask_tokens` once per chord: 1 to 10 note-steps of ~0.2 ms each.  Staging the weights, building the
+# stack plan and preparing the per-position terms of the whole window on every call would cost more than the notes, so the decoder
+# keeps a session between calls: staged weights, the stack plan with its input front, KV buffer sets of `cap` rows and the prepared
+# term buffers, all with row stride `cap`.  A call prepares the terms of its new rows only and continues a prefix the session handed
+# out in place.  The session is keyed by the decoder module (weakly) and (B, style width); a window longer than `cap` replaces it.
+_SESSIONS: "weakref.WeakKeyDictionary" = weakref.WeakKeyDictionary()
+SESSION_MIN_CAP = 256          # smallest window capacity a session is built with (capacities are powers of two up to 2048)
+SESSION_POOL = 4               # KV buffer sets a session keeps for renderings that alternate on one decoder
+
+
+def _session_for(dec, tokens: Tensor, fields: Sequence[int], k: int, style: Tensor) -> Optional["_RenderSession"]:
+    """The decoder's render session for a streaming call of this shape, or None when the note-step of the session cannot express
+    the call (the call then runs `render_decoder` as a one-off): the persistent stack kernel with its input front and the fused
+    sampling kernel must both apply."""
+    B, T, F = tokens.shape
+    S = style.shape[-1]
+    if not tokens.is_cuda or K._os.environ.get("SPB_DECODE", "fused") != "fused":
+        return None
+    tr, sizes = dec.transformer, dec.token_emb.field_sizes
+    hidden = tr.layers[1][1].ff[3].weight.shape[1]
+    if not K.decode_stack_ok(tr.depth, tr.dim, tr.heads, hidden, tr.ada_norm, S, T):
+        return None
+    cap = max(SESSION_MIN_CAP, 1 << (T - 1).bit_length())
+    if (B * cap * (2 * tr.depth + 1) * 512 * 2 > ADALN_TERMS_MAX_BYTES or len(sizes) * 128 != 1536 or dec.dim != 256
+            or dec.lm_head.split_dims[0] != 128 or len(fields) > 8 or any(sizes[f] > 256 for f in fields) or not 1 <= k <= 32):
+        return None
+    per_shape = _SESSIONS.setdefault(dec, {})
+    session = per_shape.get((B, S))
+    if session is None or session.cap < T:
+        session = per_shape[(B, S)] = _RenderSession(dec, B, S, min(cap, 2048), tokens.device)
+    return session
+
+
+class _KVSet:
+    """One set of per-layer KV buffers [B, cap, 128] of a render session, with weak references to the caches handed out from it."""
+
+    def __init__(self, depth: int, B: int, cap: int, dev):
+        self.kv = [torch.zeros((B, cap, 128), dtype=BF16, device=dev) for _ in range(depth)]
+        self._bases = {kv.untyped_storage().data_ptr() for kv in self.kv}
+        self.handed: List[weakref.ref] = []
+
+    def rows_in_use(self) -> int:
+        """The end row of the longest prefix an alive cache object handed out from this set still views (0: the set is free)."""
+        rows, alive = 0, []
+        for ref in self.handed:
+            c = ref()
+            if c is None:
+                continue
+            alive.append(ref)
+            for a in (c.transformer.attention or []) if c.transformer is not None else []:
+                for t in (a.keys, a.values):
+                    if t is not None and t.dim() == 3 and t.untyped_storage().data_ptr() in self._bases:
+                        rows = max(rows, (t.storage_offset() % t.stride(0)) // 128 + t.shape[1])
+        self.handed = alive
+        return rows
+
+    def holds_prefix(self, att, start: int) -> bool:
+        """Whether `att` are exactly rows [0, start) of this set's buffers (the caches of a call this set served, cut from the right)."""
+        for a, kv in zip(att, self.kv):
+            k, v = a.keys, a.values
+            if k.shape != (kv.shape[0], start, 64) or v.shape != k.shape or k.stride() != kv.stride() or v.stride() != kv.stride():
+                return False
+            if k.data_ptr() != kv.data_ptr() or v.data_ptr() != kv.data_ptr() + 64 * kv.element_size():
+                return False
+        return True
+
+
+class _RenderSession:
+    """Streaming calls of `unmask_mixlm` on one decoder for one (B, style width, capacity); see the comment above `_SESSIONS`.
+
+    Staleness: every call starts with session_begin (csrc/decode_stack.cu), which hashes all parameters and buffers of the decoder
+    on the device and compares the fingerprint with the one of the staged weights; the host reads the flag (one 8-byte copy) and
+    restages if it is set or if the parameters' addresses changed.  The fingerprint catches what torch's version counters miss: the
+    flat AdamW kernel of TrainStep, `p.data` edits, `load_state_dict`."""
+
+    def __init__(self, dec, B: int, S: int, cap: int, dev):
+        tr = dec.transformer
+        self.B, self.S, self.cap, self.depth, self.dim = B, S, cap, tr.depth, dec.dim
+        F = len(dec.token_emb.field_sizes)
+        D, n_gb = dec.dim, (2 * tr.depth + 1) * 512
+        self.P2 = torch.empty((B, cap, D), dtype=F32, device=dev)
+        self.C2 = torch.empty((B, cap, D), dtype=F32, device=dev)
+        self.gb_all = torch.empty((B, cap, n_gb), dtype=BF16, device=dev)
+        self.tok = torch.zeros((B, cap, F), dtype=torch.int64, device=dev)
+        self.mask = torch.ones((B, cap), dtype=torch.bool, device=dev)
+        self.zeros = torch.zeros((B, cap, D), dtype=F32, device=dev)       # token_emb / hiddens placeholders of the returned caches
+        self.tok_buf = torch.empty((B, F), dtype=torch.int64, device=dev)
+        self.p2_buf = torch.empty((B, D), dtype=F32, device=dev)
+        self.c2_buf = torch.empty((B, D), dtype=F32, device=dev)
+        self.x1_buf = torch.empty((B, F * 128), dtype=BF16, device=dev)
+        self.pos_t = torch.zeros(1, dtype=torch.int64, device=dev)
+        self.advance = torch.zeros(2, dtype=torch.int32, device=dev)
+        self.state = torch.zeros(4, dtype=torch.int64, device=dev)          # session_begin: fingerprint, 2 scratch words, stale flag
+        self.sets: List[_KVSet] = [_KVSet(tr.depth, B, cap, dev)]
+        self.w: Optional[_DecoderWeights] = None
+        self.plan: Optional[K.DecodeStackPlan] = None
+        self._ptrs: Optional[Tuple[int, ...]] = None
+        self._table: Optional[Tensor] = None
+        self.restages = 0
+
+    def _stage(self, dec) -> None:
+        w = _DecoderWeights(dec)
+        sw = w.sw
+        self.w_comp16, b_comp = w.compose_front()
+        self.b_p2 = w.bm + b_comp
+        self.plan = K.DecodeStackPlan(sw.layers, sw.w_ada, sw.b_ada, self.sets[0].kv, self.B, self.S, advance=self.advance)
+        self.plan.set_front(self.x1_buf, self.w_comp16, self.p2_buf, w.en_w.float().contiguous(), w.en_b.float().contiguous(),
+                            w.wc_l.t().contiguous(), self.c2_buf)
+        self.w = w
+        self.restages += 1
+
+    def _kv_set(self, att, start: int) -> _KVSet:
+        """The buffer set this call writes rows >= start of: the set `att` is a prefix of when no other alive cache of it reaches
+        beyond `start`, else a free set (allocated if none) that the prefix is copied into."""
+        if start > 0:
+            for s in self.sets:
+                if s.holds_prefix(att, start) and s.rows_in_use() <= start:
+                    return s
+        free = next((s for s in self.sets if s.rows_in_use() == 0), None)
+        if free is None:
+            free = _KVSet(self.depth, self.B, self.cap, self.P2.device)
+            self.sets.append(free)
+            if len(self.sets) > SESSION_POOL:      # forgetting a set never overwrites it: its caches keep their buffers alive
+                self.sets.pop(0)
+        for a, kv in zip(att, free.kv):
+            kv[:, :start, :64] = a.keys
+            kv[:, :start, 64:] = a.values
+        return free
+
+    def render(self, dec, perf: Tensor, masked_perf: Tensor, context: Tensor, style: Tensor, mask: Optional[Tensor],
+               fields: Sequence[int], temperature: float, k: int, start: int, caches):
+        """`render_decoder(start=start, kv_init=keys | values of caches, return_kv=True, use_graph=False)` plus the caches in the
+        reference's layout, with the same tokens and keys / values."""
+        B, T, F = perf.shape
+        s, n = start, T - start
+        sizes = dec.token_emb.field_sizes
+        tensors = list(dec.parameters()) + list(dec.buffers())
+        ptrs = tuple(t.data_ptr() for t in tensors)
+        if ptrs != self._ptrs:                     # `.to()`, re-allocation: hash the new tensors, restage below
+            self._table, self._ptrs, self.w = K.fingerprint_table([t.detach() for t in tensors]), ptrs, None
+        K.session_begin(self._table, self.state, self.advance, self.pos_t, s)
+        if bool(self.state[3].item()) or self.w is None:
+            self._stage(dec)
+        w, plan, Dm = self.w, self.plan, self.dim
+        seed = K.seed_from_torch() if k > 1 else 0
+        kvset = self._kv_set(caches.transformer.attention if s > 0 else [], s)
+        plan.set_kv(kvset.kv)
+
+        # the per-position terms of the new rows s..T-1 (a row of these launches does not depend on the other rows)
+        self.tok[:, s:T] = perf[:, s:T]
+        km = None
+        if mask is not None:
+            self.mask[:, :T] = mask
+            km = self.mask
+        x2, _, _ = K.embed_ln_fwd(masked_perf[:, s:T].reshape(-1, F), w.table, sizes, w.ln_w, w.ln_b)
+        x2p = K.gemm(x2, w.wp16, bias=w.bp, out_dtype=BF16)
+        self.P2[:, s:T] = K.gemm(x2p, w.wm_r, bias=self.b_p2, out_dtype=F32).view(B, n, Dm)
+        ctx16 = K.cast_bf16(context[:, s:T].float().contiguous().view(B * n, -1))
+        self.C2[:, s:T] = K.gemm(ctx16, w.wc_r, bias=w.bc, out_dtype=F32).view(B, n, Dm)
+        self.gb_all[:, s:T] = plan.prepare_adaln(style[:, s:T].float().contiguous())
+
+        offs, vocab, ks = [w.offs[f] for f in fields], [sizes[f] for f in fields], [k] * len(fields)
+        gather_src, gather_dst = [self.tok, self.P2, self.C2], [self.tok_buf, self.p2_buf, self.c2_buf]
+        for _ in range(T - 1 - s):
+            # the note-step of render_decoder with the stack kernel, its input front and the sampling kernel that ends the step
+            K.gather_at_pos(gather_src, gather_dst, [0, 1, 1], self.pos_t)
+            K.embed_ln_fwd(self.tok_buf, w.table, sizes, w.ln_w, w.ln_b, out=self.x1_buf)
+            plan.step(None, None, km, self.pos_t, gb_all=self.gb_all, use_front=True, barrier_is_zero=True)
+            e_raw = K.gemm(plan.out16, w.whead16, trans_b=True, out_dtype=BF16)
+            e, _, _ = K.layer_norm_fwd(e_raw, w.hn_w, w.hn_b, out_dtype=BF16, need_stats=False)
+            K.sample_fields(e, w.table16, fields, offs, vocab, ks, self.tok, self.pos_t, temperature=temperature, seed=seed,
+                            advance=plan.advance)
+        res = perf.clone()
+        res[:, s + 1:T] = self.tok[:, s + 1:T]
+        out_caches = _kv_only_caches(dec, kvset.kv, T - 1, zeros=self.zeros)
+        kvset.handed.append(weakref.ref(out_caches))
+        return res, out_caches
 
 
 def _unmask_stepwise(wrapper, out, tokens_masked, mask, notes, hit, temperature, filter_logits_fn, filter_kwargs, filter_key_ids, caches, kwargs):

@@ -154,7 +154,8 @@ def layer_norm_bwd(dy: Tensor, x: Tensor, mean: Tensor, rstd: Tensor, w: Optiona
 class DecodeStackPlan:
     """Pointer table + scratch of `spb_decode_stack_step` for one (stack, batch, cache) -- built once per decode session."""
 
-    def __init__(self, layers, w_ada: Tensor, b_ada: Tensor, kv_caches, B: int, style_dim: int, keep_hiddens: bool = False):
+    def __init__(self, layers, w_ada: Tensor, b_ada: Tensor, kv_caches, B: int, style_dim: int, keep_hiddens: bool = False,
+                 advance: Optional[Tensor] = None):
         import ctypes
         dev = w_ada.device
         self.depth, self.B, self.S, self.cap = len(layers), B, style_dim, kv_caches[0].shape[1]
@@ -181,8 +182,20 @@ class DecodeStackPlan:
         self.out16 = torch.empty((B, 256), dtype=BF16, device=dev)          # bf16 copy of `out`: the head projection's operand
         self._no_style = torch.zeros((B, style_dim), dtype=F32, device=dev)   # placeholder when the AdaLN terms are prepared ahead
         self._front = None
-        self.advance = torch.zeros(2, dtype=torch.int32, device=dev)         # [CTA counter of sample_fields, grid-barrier word]
+        # [CTA counter of sample_fields, grid-barrier word]; a render session passes its own, which session_begin clears every call
+        if advance is None:
+            advance = torch.zeros(2, dtype=torch.int32, device=dev)
+        assert advance.dtype == torch.int32 and advance.shape == (2,) and advance.is_contiguous()
+        self.advance = advance
         self.barrier = self.advance[1:]
+
+    def set_kv(self, kv_caches) -> None:
+        """Point the plan at another set of KV buffers of the same shape (the buffer sets of a render session)."""
+        assert len(kv_caches) == self.depth
+        for l, kv in enumerate(kv_caches):
+            assert kv.dtype == BF16 and kv.is_contiguous() and kv.shape == (self.B, self.cap, 128)
+            self.ptrs[9 * l + 6] = kv.data_ptr()
+        self._keep[1] = kv_caches
 
     def prepare_adaln(self, style_all: Tensor) -> Tensor:
         """(gamma-1 | beta) rows of every AdaLN for ALL positions, style_all fp32 [B, T, S] -> bf16 [B, T, (2*depth+1)*512]: one
@@ -279,6 +292,31 @@ def sample_fields(e: Tensor, table16: Tensor, fields: Sequence[int], offsets: Se
                     words[8 * i + v // 32] |= 1 << (v % 32)
             bits = (ctypes.c_uint32 * (8 * n))(*words)
         _call("spb_sample_fields_filtered", *args, farr(pp), farr(a_pow), farr(a_ratio), bits, _stream())
+    _count()
+
+
+def fingerprint_table(tensors: Sequence[Tensor]) -> Tensor:
+    """The [n, 3] int64 table session_begin hashes: (address, number of 32-bit words, index of the first word) per tensor, in order.
+    Returned on the tensors' device.  Every tensor must be contiguous and a whole number of 4-byte-aligned words."""
+    rows, first = [], 0
+    for t in tensors:
+        nbytes = t.numel() * t.element_size()
+        if not t.is_contiguous() or nbytes % 4 or t.data_ptr() % 4:
+            raise ValueError(f"fingerprint_table: needs contiguous tensors of whole 32-bit words, got {t.dtype} {tuple(t.shape)}")
+        rows.append((t.data_ptr(), nbytes // 4, first))
+        first += nbytes // 4
+    return torch.tensor(rows, dtype=torch.int64).reshape(-1, 3).to(tensors[0].device if len(tensors) else "cpu")
+
+
+def session_begin(table: Tensor, state: Tensor, advance: Tensor, pos_dev: Tensor, start: int) -> None:
+    """One launch at the start of a render session's call (csrc/decode_stack.cu): fingerprint of the tensors in `table`
+    (fingerprint_table) -> state[0], state[3] = 1 if it differs from the state[0] stored before, else 0; advance[:] = 0; pos_dev = start.
+    state: int64 [4] (the kernel works on it as uint64), [1] and [2] zero between launches."""
+    _require_cuda(table, state, advance, pos_dev)
+    assert table.dtype == torch.int64 and table.dim() == 2 and table.shape[1] == 3 and table.is_contiguous()
+    assert state.dtype == torch.int64 and state.shape == (4,) and state.is_contiguous()
+    assert advance.dtype == torch.int32 and advance.shape == (2,) and pos_dev.dtype == torch.int64 and pos_dev.numel() == 1
+    _call("spb_session_begin", _p(table), table.shape[0], _p(state), _p(advance), _p(pos_dev), int(start), _stream())
     _count()
 
 

@@ -32,6 +32,7 @@ SIGNATURES = {
     "spb_sample_fields_filtered": [_P, _I, _P, _P, _P, _P, _P, _I, _I, _F, _U64, _P, _P, _I, _I, _I, _P, _P, _P, _P, _P, _P],
     "spb_decode_stack_step": [_P, _P, _I, _P, _P, _P, _I, _P, _P, _I, _I, _P, _P, _P, _P, _P, _P, _P, _P, _P, _F, _P, _I, _P, _I, _P],
     "spb_gather_at_pos": [_P, _P, _P, _P, _I, _P, _I, _I, _P],
+    "spb_session_begin": [_P, _I, _P, _P, _P, c_longlong, _P],
     "spb_unpack_batch": [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _U32, _U32, _I, c_longlong, _I, _P],
     "spb_ffn_fwd": [_P, _I, _P, _P, _P, _P, _I, _P, _I, _P, _P, _I, _I, _I, _F, _U64, _P, _P],
     "spb_ffn_bwd": [_P, _I, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _F, _U64, _P, _P],
